@@ -5,6 +5,8 @@ per-pair match counts).
 
     python bench.py [--gpus N --steps K --warmup W] [--workload cfg1|cfg2|cfg3|cfg4]   # this repo's CUDA path
     python bench.py --impl reference [...]                                             # CPU baseline (oracle port)
+    python bench.py [...] --dump-outputs DIR      # also write what the last timed step returned, DIR/<name>.npy
+
 
 Workloads (BASELINE.json `configs`; per GPU, weak scaling):
     cfg1  64 pairs x 128 lines x 21 tokens x d256        (the headline configuration, default)
@@ -12,7 +14,7 @@ Workloads (BASELINE.json `configs`; per GPU, weak scaling):
     cfg3  64 pairs, ragged 32..512 lines/image, 64 token slots, 5..64 real tokens/line (256 pairs over 4 GPUs)
     cfg4  matcher only: 64 pairs x (1024 x 1024) x d256
 
-Prints ONE JSON line (contract in the task statement): `value` = pairs/s with inputs resident in
+Prints ONE JSON line: `value` = pairs/s with inputs resident in
 HBM, `e2e` = the same through pinned-host buffers (H2D of every input tensor and D2H of the match
 indices inside the timed region), `roofline` for the dominant kernel class (a second pass of the same
 K steps with a CUDA-event pair around every launch on the launching stream; separate so that the
@@ -165,6 +167,30 @@ def load_weights():
     return syn.make_state_dict(0, 1), "random-init weights (seeded)"
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: device tensor} as out_dir/<name>.npy: floating outputs as float32, integer ones as float64
+    (exact).  Beyond DUMP_BUDGET_BYTES in all, every array is cut to the same fixed, seeded sample of its
+    elements, whose flat indices go to <name>_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().cpu().numpy().reshape(-1) for k, v in arrays.items()}
+    host = {k: v.astype(np.float32 if v.dtype.kind == "f" else np.float64) for k, v in host.items()}
+    frac = None
+    if sum(v.nbytes for v in host.values()) > DUMP_BUDGET_BYTES:
+        # a sampled element costs its value plus its float64 index; 4 KB per file for the two .npy headers
+        cost = sum(v.size * (v.itemsize + 8) for v in host.values())
+        frac = (DUMP_BUDGET_BYTES - 2 * 4096 * len(host)) / cost
+    for k, v in host.items():
+        if frac is not None:
+            n = int(v.size * frac)
+            idx = np.sort(np.random.Generator(np.random.PCG64(0)).choice(v.size, size=n, replace=False))
+            np.save(os.path.join(out_dir, f"{k}_index.npy"), idx.astype(np.float64))
+            v = v[idx]
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+
+
 def cfg3_sizes(seed, n):
     rng = np.random.Generator(np.random.PCG64(seed))
     return [int(x) for x in rng.integers(32, 513, size=n)]
@@ -293,11 +319,15 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=4, help="pair groups whose H2D copy overlaps compute in the e2e leg")
     ap.add_argument("--profile-only", action="store_true", help="resident steps only (for runs under ncu)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank r > 0: <name>_rank<r>.npy)")
     ap.add_argument("--cpu-worker", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--threads", type=int, default=1, help=argparse.SUPPRESS)
     ap.add_argument("--n", type=int, default=10, help=argparse.SUPPRESS)
     ap.add_argument("--warm", type=int, default=3, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.cpu_worker:
         return cpu_worker(args)
     rank, world = env_int("RANK", 0), env_int("WORLD_SIZE", 1)
@@ -390,31 +420,33 @@ def main():
             gathered["last"] = h.result() if peer is not None else h.wait()
 
     def run_resident(gather=None):
+        """-> the arrays the caller of the path receives (on the device)."""
         if wl == "cfg4":
             out = _ops.match_descriptors(res0, res1, _native.LAYOUT_ROWS, P, 0.8, True, n0=1024, n1=1024, want_dist=False,
                                          gather=gather)
-            return out["matches0"], out["counts"]
+            return {k: out[k] for k in ("matches0", "scores0", "nn1", "counts")}
         res = eng.match_packed(resident, P, 0.8, gather=gather)
-        return res.matches0, res.counts
+        return {"matches0": res.matches0, "scores0": res.scores0, "counts": res.counts,
+                "offsets0": torch.from_numpy(res.offsets0)}
 
     def step_resident():
         if peer is not None:
-            m0, cnt = run_resident(peer.publish())
+            out = run_resident(peer.publish())
             # counts of step i-2: one exchange stays in flight across the step boundary.  A host that waits for the
             # previous step's counts (and the peers' flags) before it enqueues the next step lets the launch queue run dry
             # whenever the ranks drift into ping-pong - the same box measured 0.99 and 1.41 ms per step that way.  With
             # LTR_GATHER_SLOTS = 8 a peer can only overwrite a slot 8 steps later, when this rank has long read it.
             drain(max(KEEP, 1))
             pending.append((None, peer.collect_async())) # copy-engine D2H of this step's slot behind this step's kernels
-            return m0, cnt
-        m0, cnt = run_resident()
+            return out
+        out = run_resident()
         if world > 1 and gather_mode != "off":
             # NCCL path: one all-gather stays in flight across the step boundary - its kernel has to find an SM between
             # persistent CTAs that follow each other without a gap (PDL), and a host that waits for it every step lets
             # the launch queue run dry (measured 1.41 ms per step against 1.05 ms)
             drain(max(KEEP, 1))
-            pending.append(gather_counts(cnt, P * world, async_op=True))
-        return m0, cnt
+            pending.append(gather_counts(out["counts"], P * world, async_op=True))
+        return out
 
     out_host = {"m": torch.empty(n_out, dtype=torch.int32).pin_memory(), "c": torch.empty(P, dtype=torch.int32).pin_memory()}
 
@@ -442,7 +474,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        timed_out = step_resident()
     drain()            # the last step's all-gather is inside the timed region
     e1.record()
     barrier()
@@ -454,10 +486,14 @@ def main():
     #      kernels serialises them and would switch off the programmatic dependent launch overlap. ----
     _native.profile_begin()
     for _ in range(args.steps):
-        m_last, c_last = step_resident()
+        last = step_resident()
     drain()
     barrier()
     prof = _native.profile_end()
+    m_last, c_last = last["matches0"], last["counts"]
+    if args.dump_outputs:
+        sfx = f"_rank{rank}" if rank else ""
+        dump_outputs(args.dump_outputs, {k + sfx: v for k, v in timed_out.items()})
 
     if args.profile_only:
         return

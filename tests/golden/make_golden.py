@@ -1,11 +1,12 @@
-"""Generate golden fixtures by running the UNMODIFIED reference (imported read-only
-from /root/reference) on seeded inputs.  Run in the build container only:
+"""Generate golden fixtures by running the UNMODIFIED reference (a checkout of it, imported
+read-only) on seeded inputs:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 Inputs and synthetic weights are regenerable from seeds (linetr_b200/synthetic.py), so the
 fixtures store only the reference OUTPUTS plus input checksums that detect generator
-drift.  The reference is executed on CPU, eval mode, no grad (SURVEY.md §8c/§8d).
+drift.  The reference is executed on CPU, eval mode, no grad (SURVEY.md §8c/§8d).  The cases with the
+shipped checkpoint live in make_standin_golden.py.
 """
 import json
 import os
@@ -17,7 +18,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = os.environ.get("LINETR_REFERENCE", "/root/reference")
+REF = os.path.abspath(sys.argv[1]) if len(sys.argv) == 2 else sys.exit(__doc__)
 sys.path.insert(0, REF)
 
 from linetr_b200 import synthetic as syn  # noqa: E402
@@ -27,7 +28,6 @@ from models.nn_matcher import nn_matcher as ref_nn_matcher  # noqa: E402
 from models.nn_matcher import nn_matcher_distmat as ref_nn_matcher_distmat  # noqa: E402
 
 torch.set_grad_enabled(False)
-REAL_WEIGHTS = os.path.join(REF, "models/weights/LineTR_weight.pth")
 
 
 def checksum(d):
@@ -130,24 +130,6 @@ def main():
     out["s2k_mat"] = ref_nn_matcher_distmat(dk, 0.8, is_mutual_NN=True)
     meta["cases"]["s2k"] = {"seed": 53, "nsub0": nsub0, "nsub1": nsub1}
 
-    # ---- shipped checkpoint ----------------------------------------------------------------
-    if os.path.exists(REAL_WEIGHTS):
-        sdr = {k: v.numpy() for k, v in torch.load(REAL_WEIGHTS).items()}
-        mr = ref_model(sdr, 1)
-        d = syn.make_image_inputs(61, 16, 21, (3, 21))
-        out["real_enc_L16_T21"] = run_forward(mr, d)
-        meta["cases"]["real_enc_L16_T21"] = {"seed": 61, "L": 16, "T": 21, "ntok": (3, 21),
-                                             "weights": "shipped", "checksum": checksum(d)}
-        a, b, perm = syn.make_pair_inputs(62, 128, 21)
-        d0, d1, dk, mat = run_pair(mr, a, b, 0.8)
-        out["real_pair_L128_d0"], out["real_pair_L128_d1"] = d0, d1
-        out["real_pair_L128_mat_idx"] = np.where(mat[0].sum(1) > 0, mat[0].argmax(1), -1).astype(np.int32)
-        srt = np.sort(dk[0], axis=1)
-        meta["cases"]["real_pair_L128"] = {"seed": 62, "L": 128, "T": 21, "thr": 0.8, "weights": "shipped",
-                                           "n_matches": int(mat.sum()),
-                                           "min_top2_gap": float((srt[:, 1] - srt[:, 0]).min()),
-                                           "weights_checksum": float(sum(np.asarray(v, np.float64).sum() for v in sdr.values()))}
-
     np.savez_compressed(os.path.join(HERE, "reference_outputs.npz"), **out)
     with open(os.path.join(HERE, "reference_outputs.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
@@ -155,27 +137,5 @@ def main():
           {k: v.get("n_matches") for k, v in meta["cases"].items() if "n_matches" in v})
 
 
-def main_full():
-    """Full-size images of BASELINE.json's cfg[2] / cfg[3] shapes through the unmodified reference with the shipped
-    checkpoint: 256 lines x 32 tokens, and 512 lines x 64 tokens with ragged real-token counts.  Separate fixture
-    file (outputs only, ~0.7 MB): `reference_outputs_full.npz|json`."""
-    out, meta = {}, {"torch": torch.__version__, "numpy": np.__version__, "cases": {}}
-    sdr = {k: v.numpy() for k, v in torch.load(REAL_WEIGHTS).items()}
-    mr = ref_model(sdr, 1)
-    for name, c in {"real_enc_L256_T32": dict(seed=71, L=256, T=32, ntok=None),
-                    "real_enc_L512_T64_ragged": dict(seed=72, L=512, T=64, ntok=(3, 64))}.items():
-        d = syn.make_image_inputs(c["seed"], c["L"], c["T"], c["ntok"])
-        out[name] = run_forward(mr, d)
-        meta["cases"][name] = {**c, "weights": "shipped", "checksum": checksum(d)}
-        print(name, out[name].shape)
-    np.savez_compressed(os.path.join(HERE, "reference_outputs_full.npz"), **out)
-    with open(os.path.join(HERE, "reference_outputs_full.json"), "w") as f:
-        json.dump(meta, f, indent=1, sort_keys=True)
-
-
 if __name__ == "__main__":
-    if "--full-only" in sys.argv:
-        main_full()
-    else:
-        main()
-        main_full()
+    main()

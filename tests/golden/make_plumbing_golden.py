@@ -1,8 +1,8 @@
 """cfg[0] plumbing fixtures: run the UNMODIFIED reference `Matching` (models/matching.py) on the four
 bundled image pairs (assets/input_pairs.txt) exactly as match_line_pairs.py configures it, on CPU,
-and commit what the hot path received and produced.  Build container only:
+and commit what the hot path received and produced.  Needs a checkout of the reference:
 
-    python tests/golden/make_plumbing_golden.py
+    python tests/golden/make_plumbing_golden.py <reference checkout>
 
 The reference's LSD wrapper needs opencv-contrib's `cv2.line_descriptor` (absent here, SURVEY.md 8c):
 a TEST-ONLY shim detector built on the main-module `cv2.createLineSegmentDetector` stands in.  Which
@@ -11,16 +11,20 @@ dict - but the tokeniser, LineTransformer.forward, get_dist_matrix, subline2keyl
 nn_matcher_distmat calls are the reference's own, with real SuperPoint descriptors, real line
 geometry, real key-line -> subline splits (mat_klines2sublines is not the identity).
 
-Stored per image (fixture `plumbing_pairs.npz`): the tokeniser dict (descriptors of padded token
+The line transformer keeps the MAX_KEYLINES strongest key lines of each image (the reference's own
+`max_keylines` option; every other setting is match_line_pairs.py's), which keeps each fixture file well
+under 1 MB.  Stored per image (fixture `plumbing_pairs_p<i>.npz`, one file per pair): the tokeniser dict (descriptors of padded token
 slots are all the descriptor sampled at (0, 0), so only real-token descriptors + that one pad
 descriptor are stored and `tests/helpers.plumbing_image` rebuilds the tensor bit-exactly) and the
 reference outputs `line_desc`, `matches_l`, `matching_scores_l`; for one pair also the SuperPoint point
-descriptors + `matches_p` (the nn_matcher call of matching.py:69-71).
+descriptors + `matches_p` (the nn_matcher call of matching.py:69-71, `plumbing_points.npz`).
 Also writes tokenizer fixtures (`tokenizer_outputs.npz`): outputs of the reference tokeniser
 (`LineTransformer.preprocess`, models/line_transformer.py:251-275 -> models/line_process.py:100-196) for the seeded
 fake detections / fake SuperPoint maps of tests/test_tokenizer.py, so that the GPU tokenizer is
-checked against REFERENCE data on the GPU box (where /root/reference does not exist).
+checked against REFERENCE data.  `desc_sublines` is stored as the SHA-256 of its bytes (bit-identity checks),
+its shape and DESC_SAMPLE seeded token rows (tolerance checks).
 """
+import hashlib
 import json
 import os
 import sys
@@ -32,10 +36,10 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get("LINETR_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
-sys.path.insert(0, REF)
 torch.set_grad_enabled(False)
+MAX_KEYLINES = 20
+DESC_SAMPLE = 64
 
 
 class ShimKeyLine:
@@ -64,12 +68,12 @@ class ShimLSD:
 
 
 def reference_matching_config():
-    """The config dict match_line_pairs.py:54-73 builds (defaults of its argparse)."""
+    """The config dict match_line_pairs.py:54-73 builds (defaults of its argparse), MAX_KEYLINES key lines."""
     return {
         "auto_min_length": True,
         "superpoint": {"nms_radius": 4, "keypoint_threshold": 0.005, "max_keypoints": 1024, "nn_threshold": 0.7},
         "lsd": {"n_octave": 2},
-        "linetransformer": {"max_keylines": -1, "min_length": 16, "token_distance": 8, "nn_threshold": 0.8},
+        "linetransformer": {"max_keylines": MAX_KEYLINES, "min_length": 16, "token_distance": 8, "nn_threshold": 0.8},
     }
 
 
@@ -101,16 +105,18 @@ def pack_image(out, prefix, pred, side):
     out[f"{prefix}_line_desc"] = g("line_desc")
 
 
-def main():
+def main(ref):
+    sys.path.insert(0, ref)
     import models.matching as ref_matching
     ref_matching.LSD = ShimLSD                       # the only substitution; everything else is stock
     matching = ref_matching.Matching(reference_matching_config()).eval()
-    with open(os.path.join(REF, "assets", "input_pairs.txt")) as f:
+    with open(os.path.join(ref, "assets", "input_pairs.txt")) as f:
         pairs = [l.split()[:2] for l in f.readlines() if l.strip()]
-    out, meta = {}, {"pairs": []}
+    meta = {"pairs": [], "max_keylines": MAX_KEYLINES}
     for i, (n0, n1) in enumerate(pairs):
-        im0 = read_image(os.path.join(REF, "assets", n0))
-        im1 = read_image(os.path.join(REF, "assets", n1))
+        out = {}
+        im0 = read_image(os.path.join(ref, "assets", n0))
+        im1 = read_image(os.path.join(ref, "assets", n1))
         pred = matching({"image0": im0, "image1": im1})
         pack_image(out, f"p{i}_0", pred, "0")
         pack_image(out, f"p{i}_1", pred, "1")
@@ -125,13 +131,13 @@ def main():
         srt = np.sort(d, axis=1)
         info["min_top2_gap_rows"] = float((srt[:, 1] - srt[:, 0]).min())
         if i == 0:   # point branch (matching.py:69-71): descriptors [256, N] + the reference's matches
-            out["p0_desc_pnt0"] = pred["descriptors0"][0].numpy()
-            out["p0_desc_pnt1"] = pred["descriptors1"][0].numpy()
-            out["p0_matches_p"] = np.where(pred["matches_p"][0].numpy().sum(1) > 0,
-                                           pred["matches_p"][0].numpy().argmax(1), -1).astype(np.int32)
+            np.savez_compressed(os.path.join(HERE, "plumbing_points.npz"), p0_desc_pnt0=pred["descriptors0"][0].numpy(),
+                                p0_desc_pnt1=pred["descriptors1"][0].numpy(),
+                                p0_matches_p=np.where(pred["matches_p"][0].numpy().sum(1) > 0,
+                                                      pred["matches_p"][0].numpy().argmax(1), -1).astype(np.int32))
         meta["pairs"].append(info)
         print(info)
-    np.savez_compressed(os.path.join(HERE, "plumbing_pairs.npz"), **out)
+        np.savez_compressed(os.path.join(HERE, f"plumbing_pairs_p{i}.npz"), **out)
     meta["torch"] = torch.__version__
     meta["note"] = "reference Matching (CPU) with a cv2.createLineSegmentDetector shim for the LSD wrapper"
 
@@ -147,10 +153,12 @@ def main():
         for k, v in want.items():
             a = v.numpy()
             if k == "desc_sublines":
-                mask = want["mask_sublines"][0, :, 1:, 0].numpy() > 0
-                tok[f"c{ci}_desc_real"] = a[0][mask]
-                pads = a[0][~mask]
-                tok[f"c{ci}_desc_pad"] = pads[0] if len(pads) else np.zeros(256, np.float32)
+                a = np.ascontiguousarray(a)
+                tok[f"c{ci}_desc_sha256"] = np.frombuffer(hashlib.sha256(a.tobytes()).digest(), np.uint8)
+                tok[f"c{ci}_desc_shape"] = np.array(a.shape, np.int64)
+                flat = a.reshape(-1, a.shape[-1])
+                rows = np.sort(np.random.Generator(np.random.PCG64(ci)).choice(len(flat), DESC_SAMPLE, replace=False))
+                tok[f"c{ci}_desc_rows"], tok[f"c{ci}_desc_sample"] = rows, flat[rows]
             else:
                 tok[f"c{ci}_{k}"] = a
     meta["tokenizer_cfgs"] = cfgs
@@ -176,9 +184,12 @@ def main():
     np.savez_compressed(os.path.join(HERE, "tokenizer_outputs.npz"), **tok)
     with open(os.path.join(HERE, "plumbing_pairs.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
-    for fn in ("plumbing_pairs.npz", "tokenizer_outputs.npz", "eval_matcher_outputs.npz"):
-        print(fn, os.path.getsize(os.path.join(HERE, fn)) / 1e6, "MB")
+    for fn in sorted(os.listdir(HERE)):
+        if fn.endswith(".npz"):
+            print(fn, os.path.getsize(os.path.join(HERE, fn)) / 1e6, "MB")
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(os.path.abspath(sys.argv[1]))

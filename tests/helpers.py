@@ -18,17 +18,7 @@ def golden():
     return _cache["npz"], _cache["meta"]
 
 
-def golden_full():
-    """Full-size images (256 x 32, ragged 512 x 64) through the reference with the shipped checkpoint
-    (tests/golden/make_golden.py::main_full)."""
-    if "npz_full" not in _cache:
-        _cache["npz_full"] = dict(np.load(os.path.join(GOLDEN_DIR, "reference_outputs_full.npz")))
-        with open(os.path.join(GOLDEN_DIR, "reference_outputs_full.json")) as f:
-            _cache["meta_full"] = json.load(f)
-    return _cache["npz_full"], _cache["meta_full"]
-
-
-FULL_CASES = ["real_enc_L256_T32", "real_enc_L512_T64_ragged"]
+FULL_CASES = ["real_enc_L256_T32", "real_enc_L512_T64_ragged"]   # cases of standin()
 
 
 def checksum(d):
@@ -46,27 +36,55 @@ def weights_for(tag):
     kind, *rest = tag.split(":")
     if kind == "synthetic":
         return syn.make_state_dict(int(rest[0]), int(rest[1]))
+    if kind == "standin":
+        return standin_weights()
     raise KeyError(tag)
 
 
-def shipped_weights_path():
-    """The reference checkpoint, if a copy travelled with the repo (git-ignored) or the
-    reference checkout is mounted (build container only)."""
-    root = os.path.dirname(GOLDEN_DIR[:-len("/golden")])
-    for p in (os.environ.get("LINETR_WEIGHTS", ""),
-              os.path.join(root, "linetr_b200", "weights", "LineTR_weight.pth"),
-              "/root/reference/models/weights/LineTR_weight.pth"):
-        if p and os.path.exists(p):
-            return p
-    return None
+STANDIN_SEED = 2024
 
 
-def load_shipped_weights():
-    p = shipped_weights_path()
-    if p is None:
-        return None
+def standin_weights():
+    """Stand-in for the shipped LineTR checkpoint (22 MB, not part of the repository): every tensor is
+    seeded normal noise with the mean and standard deviation of the shipped tensor, clipped to its range
+    (golden/checkpoint_stats.json), so that BatchNorm statistics, LayerNorm gains and weight scales have
+    the trained model's magnitudes.  golden/standin_outputs.npz holds what the reference computed with it."""
+    if "standin" not in _cache:
+        with open(os.path.join(GOLDEN_DIR, "checkpoint_stats.json")) as f:
+            stats = json.load(f)
+        rng = np.random.Generator(np.random.PCG64(STANDIN_SEED))
+        sd = {}
+        for key, shape, kind in syn.state_dict_spec(1):
+            mean, std, lo, hi = stats[key]
+            if kind == "bn_count":
+                sd[key] = np.array(int(mean), dtype=np.int64)
+            else:
+                sd[key] = np.clip(mean + std * rng.standard_normal(shape), lo, hi).astype(np.float32)
+        _cache["standin"] = sd
+    return _cache["standin"]
+
+
+def save_standin_checkpoint(path):
+    """The stand-in as a checkpoint file (what LineTransformer(mode='test') loads)."""
     import torch
-    return {k: v.numpy() for k, v in torch.load(p, map_location="cpu").items()}
+    torch.save({k: torch.from_numpy(v.copy()) for k, v in standin_weights().items()}, path)
+    return str(path)
+
+
+def standin():
+    """Outputs of the reference with the stand-in checkpoint (tests/golden/make_standin_golden.py).  Large
+    descriptor sets are stored as a seeded sample of lines: `<name>_cols` indexes the lines of `<name>`."""
+    if "standin_npz" not in _cache:
+        _cache["standin_npz"] = dict(np.load(os.path.join(GOLDEN_DIR, "standin_outputs.npz")))
+        with open(os.path.join(GOLDEN_DIR, "standin_outputs.json")) as f:
+            _cache["standin_meta"] = json.load(f)
+    return _cache["standin_npz"], _cache["standin_meta"]
+
+
+def sampled(npz, name, full):
+    """(stored sample, the same lines of `full` [.., 256, L])."""
+    cols = npz[f"{name}_cols"]
+    return npz[name], full[..., cols]
 
 
 def case_inputs(case):
@@ -89,9 +107,12 @@ TOK_KEYS = ("klines", "length_klines", "angles", "sublines", "pnt_sublines", "ma
 
 
 def plumbing():
-    """Fixtures of tests/golden/make_plumbing_golden.py: the reference `Matching` run on the four bundled pairs."""
+    """Fixtures of tests/golden/make_plumbing_golden.py: the reference `Matching` run on the four bundled pairs
+    (one file per pair, the point branch in plumbing_points.npz), as one dict."""
     if "plumb" not in _cache:
-        _cache["plumb"] = dict(np.load(os.path.join(GOLDEN_DIR, "plumbing_pairs.npz")))
+        names = sorted(f for f in os.listdir(GOLDEN_DIR) if f.startswith("plumbing_pairs_p") and f.endswith(".npz"))
+        _cache["plumb"] = {k: v for f in names + ["plumbing_points.npz"]
+                           for k, v in np.load(os.path.join(GOLDEN_DIR, f)).items()}
         with open(os.path.join(GOLDEN_DIR, "plumbing_pairs.json")) as f:
             _cache["plumb_meta"] = json.load(f)
     return _cache["plumb"], _cache["plumb_meta"]
@@ -114,12 +135,26 @@ def plumbing_image(npz, prefix):
 
 
 def tokenizer_fixture(ci):
+    """The reference tokeniser's dict for tokenizer config `ci`, except `desc_sublines` (see check_tokenizer_desc)."""
     if "tok" not in _cache:
         _cache["tok"] = dict(np.load(os.path.join(GOLDEN_DIR, "tokenizer_outputs.npz")))
     npz = _cache["tok"]
-    d = {k[len(f"c{ci}_"):]: v for k, v in npz.items() if k.startswith(f"c{ci}_") and not k.startswith(f"c{ci}_desc_")}
-    d["desc_sublines"] = _rebuild_desc(d["mask_sublines"], npz[f"c{ci}_desc_real"], npz[f"c{ci}_desc_pad"])
-    return d
+    return {k[len(f"c{ci}_"):]: v for k, v in npz.items() if k.startswith(f"c{ci}_") and not k.startswith(f"c{ci}_desc_")}
+
+
+def check_tokenizer_desc(got, ci, tol=None):
+    """`desc_sublines` of tokenizer config `ci` against the reference's: float32 of the same shape, and bit-identical
+    (the SHA-256 of all its bytes) or, with `tol`, the stored sample of token rows within tol."""
+    import hashlib
+    tokenizer_fixture(ci)
+    npz = _cache["tok"]
+    got = np.ascontiguousarray(got)
+    assert got.dtype == np.float32 and got.shape == tuple(npz[f"c{ci}_desc_shape"])
+    if tol is None:
+        assert hashlib.sha256(got.tobytes()).digest() == npz[f"c{ci}_desc_sha256"].tobytes()
+    else:
+        rows = got.reshape(-1, got.shape[-1])[npz[f"c{ci}_desc_rows"]]
+        assert np.abs(rows - npz[f"c{ci}_desc_sample"]).max() < tol
 
 
 def matching_line_branch(get_dist_matrix, subline2keyline, nn_matcher_distmat, line_desc0, line_desc1, A0, A1, thr):

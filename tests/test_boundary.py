@@ -1,9 +1,9 @@
 """CPU-only checks of the drop-in boundary: module surface, state-dict contract, C-ABI
 exports, host-side glue.  No compute call is made (there is no GPU here and no fallback)."""
 import ctypes
+import json
 import os
 import re
-import sys
 
 import numpy as np
 import pytest
@@ -17,7 +17,6 @@ from linetr_b200 import engine
 from tests import helpers as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def _model(nd=1):
@@ -64,31 +63,34 @@ def test_state_dict_contract():
         _model(4).load_state_dict({k: torch.from_numpy(v) for k, v in syn.make_state_dict(3, 1).items()})
 
 
-def test_shipped_checkpoint_loads_strict():
-    p = H.shipped_weights_path()
-    if p is None:
-        pytest.skip("shipped checkpoint not available")
+def test_shipped_checkpoint_loads_strict(tmp_path):
+    with open(os.path.join(H.GOLDEN_DIR, "checkpoint_stats.json")) as f:
+        shipped_keys = list(json.load(f))            # the shipped checkpoint's keys, in its order
+    p = H.save_standin_checkpoint(tmp_path / "LineTR_weight.pth")
     m = LineTransformer({"mode": "test", "weights_path": p})
     ref = torch.load(p, map_location="cpu")
-    assert list(m.state_dict().keys()) == list(ref.keys())
+    assert list(ref.keys()) == shipped_keys
+    assert list(m.state_dict().keys()) == shipped_keys
+    for k, v in ref.items():
+        assert torch.equal(m.state_dict()[k], v), k
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not mounted")
 def test_same_keys_and_init_as_reference():
-    sys.path.insert(0, REF)
-    try:
-        from models.line_transformer import LineTransformer as Ref
-    finally:
-        sys.path.remove(REF)
-    torch.manual_seed(0)
-    r = Ref({"mode": "train", "n_line_descriptive_layers": 2})
+    """Against the reference's random init (tests/golden/reference_init.json): same keys in the same order,
+    shapes, dtypes and - same RNG consumption - the same values; same config."""
+    with open(os.path.join(H.GOLDEN_DIR, "reference_init.json")) as f:
+        want = json.load(f)
     torch.manual_seed(0)
     o = _model(2)
-    rs, os_ = r.state_dict(), o.state_dict()
-    assert list(rs.keys()) == list(os_.keys())
-    for k in rs:
-        assert torch.equal(rs[k], os_[k]), k      # same RNG consumption -> same random init
-    assert r.config == o.config
+    sd = o.state_dict()
+    assert list(sd.keys()) == [t["key"] for t in want["tensors"]]
+    for t in want["tensors"]:
+        v = sd[t["key"]]
+        assert list(v.shape) == t["shape"] and str(v.dtype) == t["dtype"], t["key"]
+        flat = v.reshape(-1).double().numpy()
+        assert flat.sum() == t["sum"], t["key"]
+        assert flat[t["idx"]].tolist() == t["values"], t["key"]
+    assert o.config == want["config"]
 
 
 def test_config_and_defaults():
