@@ -924,6 +924,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(352, 1) gemm_chain2_
       uint32_t hs = 0, unpub = 0;                   // hs: hand-overs so far; unpub: k-blocks stored but not yet published
       for (int ct = cl0; ct < n_ctiles; ct += cl_step) {
         const int mt = 2 * ct + (int)rank;
+        // With an odd tile count the rank-1 CTA of the last cluster computes a tile past the end (mt == m_tiles): it
+        // runs the whole barrier protocol (the leader's MMAs cover both CTAs' rows) but its output goes nowhere.  The
+        // last op's image may be the caller's descriptor tile image, which is only 128-row padded: a store there would
+        // land in the lo plane (hi) and past the end of the buffer (lo).
+        const bool real_tile = mt < c.m_tiles;
         for (int o = 0; o < c.n_ops; ++o) {
           const GemmImgArgs& p = c.op[o];
           const bool streamed = chain2_streamed(p);
@@ -934,9 +939,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(352, 1) gemm_chain2_
                 uint8_t* tile = smem + Cfg::OFF_STG + b * Cfg::STG_TILE;
                 mbar_wait_dl(&tile_ready[b], ph, false);
                 const size_t toff = ((size_t)mt * p.O.kblocks + p.o_kb0 + nb * 4 + kbl) * IMG_TILE_ELEMS;
-                ptx::bulk_s2g(p.O.hi + toff, tile, 16384);
-                ptx::bulk_s2g(p.O.lo + toff, tile + 16384, 16384);
-                ptx::bulk_commit();
+                if (real_tile) {
+                  ptx::bulk_s2g(p.O.hi + toff, tile, 16384);
+                  ptx::bulk_s2g(p.O.lo + toff, tile + 16384, 16384);
+                }
+                ptx::bulk_commit();                   // an empty group for a phantom tile keeps the wait counts below
                 ++unpub;
                 ptx::bulk_wait_read_all();            // the copies have read staging tile b: hand it back (the epilogue
                 ptx::mbar_arrive(&tile_free[b]);      // is filling the other tile meanwhile)
@@ -1298,7 +1305,9 @@ inline int launch_gemm_img(const GemmImgArgs& a, cudaStream_t s, int bn_hint = 0
 
 // Chain of row-local layers in one launch (see gemm_chain_kernel).  Every op: N % 256 == 0, plain A
 // (no block-diagonal slices); op i+1 must read what op i writes for the same rows only.
-// pair = true: CTA-pair engine (gemm_chain2_kernel); the images must be padded to 256 rows (ltr_api.cu carve does).
+// pair = true: CTA-pair engine (gemm_chain2_kernel); the images it reads (A, residual, addend) must be padded to 256 rows
+// (ltr_api.cu carve does).  O may be padded to 128 rows only (the caller's descriptor tile image): the store warp drops
+// the output of the phantom tile an odd tile count gives the last cluster.
 inline int launch_gemm_chain(const GemmImgArgs* ops, int n_ops, cudaStream_t s, bool pair = false) {
   if (n_ops < 1 || n_ops > CHAIN_MAX_OPS) return set_error(-1, "gemm_chain: 1..4 ops");
   if (ops[0].M <= 0) return 0;
