@@ -1,5 +1,5 @@
-// CUDA-core kernels of the line-descriptor forward that are not GEMMs: the narrow head of the LINE
-// positional encoder (the token one lives in token_fused.cuh), LayerNorm, final L2 normalisation.
+// CUDA-core kernels of the line-descriptor forward that are not GEMMs: the narrow head of the line
+// positional encoder and the final L2 normalisation of the channel-first output.
 #pragma once
 #include "act_img.cuh"
 #include "common.cuh"
@@ -7,13 +7,12 @@
 namespace ltr {
 
 // ------------------------------------------------------------------------------------
-// Narrow head of the positional encoders: IN -> 32 -> 64 -> 128, eval-BatchNorm folded,
+// Narrow head of the line positional encoder: 5 -> 32 -> 64 -> 128, eval-BatchNorm folded,
 // ReLU after each layer.  Reference: MLP() models/line_transformer.py:9-20 as used by
-// WordPositionalEncoder (:61-73, IN = 3: x, y, score) and LinePositionalEncoder (:46-50,
-// IN = 5: mid x, mid y, response, cos2t, sin2t), after normalize_keylines (:22-38).
-// One warp owns SM_ROWS rows at a time; weights live in shared memory.
+// LinePositionalEncoder (:46-50, inputs: mid x, mid y, response, cos2t, sin2t), after
+// normalize_keylines (:22-38).  One warp owns SM_ROWS rows at a time; weights live in shared memory.
 struct SmallMlpWeights {
-  const float* w1;  // [32][IN]
+  const float* w1;  // [32][5]
   const float* b1;  // [32]
   const float* w2;  // [64][32]
   const float* b2;
@@ -25,9 +24,8 @@ constexpr int SM_ROWS = 4;
 constexpr int SM_WARPS = 8;
 constexpr int SM_K2 = 32 + 4, SM_K3 = 64 + 4;  // padded leading dims (bank-conflict-free float4)
 
-template <int IN>
 struct SmallMlpSmem {
-  float w1[32 * IN];
+  float w1[32 * 5];
   float b1[32], b2[64], b3[128];
   __align__(16) float w2[64 * SM_K2];
   __align__(16) float w3[128 * SM_K3];
@@ -35,16 +33,14 @@ struct SmallMlpSmem {
   __align__(16) float h2[SM_WARPS][SM_ROWS][64];
 };
 
-// TOKEN = true : row = token, inputs pnt[row][2], score[row]
-// TOKEN = false: row = line,  inputs sublines[row][2][2], resp[row], angle[row][2]
-template <bool TOKEN>
+// row = line, inputs sublines[row][2][2] (in0), resp[row] (in1), angle[row][2] (in2)
 __global__ void __launch_bounds__(SM_WARPS * 32)
 small_mlp_kernel(SmallMlpWeights w, const float* __restrict__ in0, const float* __restrict__ in1,
                  const float* __restrict__ in2, ActImg out, int rows, float cx, float cy,
                  float scale) {
-  constexpr int IN = TOKEN ? 3 : 5;
+  constexpr int IN = 5;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  auto& S = *reinterpret_cast<SmallMlpSmem<IN>*>(smem_raw);
+  auto& S = *reinterpret_cast<SmallMlpSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   pdl_launch_dependents();
   for (int i = tid; i < 32 * IN; i += blockDim.x) S.w1[i] = w.w1[i];
@@ -64,20 +60,14 @@ small_mlp_kernel(SmallMlpWeights w, const float* __restrict__ in0, const float* 
 #pragma unroll
     for (int r = 0; r < SM_ROWS; ++r) {
       int row = min(r0 + r, rows - 1);
-      if (TOKEN) {
-        x[r][0] = (in0[2 * row] - cx) / scale;
-        x[r][1] = (in0[2 * row + 1] - cy) / scale;
-        x[r][2] = in1[row];
-      } else {
-        // normalise both end points first, then take the mid point (reference order)
-        float ax = (in0[4 * row + 0] - cx) / scale, ay = (in0[4 * row + 1] - cy) / scale;
-        float bx = (in0[4 * row + 2] - cx) / scale, by = (in0[4 * row + 3] - cy) / scale;
-        x[r][0] = (ax + bx) / 2.f;
-        x[r][1] = (ay + by) / 2.f;
-        x[r][2] = in1[row];
-        x[r][3] = in2[2 * row];
-        x[r][4] = in2[2 * row + 1];
-      }
+      // normalise both end points first, then take the mid point (reference order)
+      float ax = (in0[4 * row + 0] - cx) / scale, ay = (in0[4 * row + 1] - cy) / scale;
+      float bx = (in0[4 * row + 2] - cx) / scale, by = (in0[4 * row + 3] - cy) / scale;
+      x[r][0] = (ax + bx) / 2.f;
+      x[r][1] = (ay + by) / 2.f;
+      x[r][2] = in1[row];
+      x[r][3] = in2[2 * row];
+      x[r][4] = in2[2 * row + 1];
     }
 #pragma unroll
     for (int r = 0; r < SM_ROWS; ++r) {

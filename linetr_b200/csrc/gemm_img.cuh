@@ -495,180 +495,24 @@ __global__ void __launch_bounds__(320, 1) gemm_img_kernel(GemmImgArgs p) {
   if (warp == 1) ptx::tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
-// ---------------------------------------------------------------- chained GEMMs (one launch, several row-local layers)
+// ---------------------------------------------------------------- chained GEMMs (one launch, several row-local layers, CTA pairs)
 // Layers whose inputs are row-local (every output row depends only on the same row of the previous layer's
 // output) can run back to back inside ONE persistent launch: a CTA owns a 128-row m-tile and walks through
 // all n-blocks of op 0, then of op 1, ... for that m-tile.  Compared with one launch per layer this removes
 // the per-launch fill / drain / wave-quantisation bubbles (mlp1: 256 tiles and mlp2: 128 tiles on 148 SMs
 // are 2 resp. 0.86 waves; chained, 128 CTAs do 3 + 3 tiles each) - the signature layer's
 //   mlp1 (ReLU) -> mlp2 (+ residual) -> qkv of the NEXT layer (or final_proj + L2 norm)
-// chain (models/line_transformer.py:157-166,176-183,245-246) is one launch instead of three.
-// Dependency between consecutive ops of an m-tile: the producer warp waits on `op_done` until all eight
-// epilogue warps have finished (and fenced: generic-proxy global stores -> async-proxy TMA reads) the
-// previous op's tiles of this m-tile.  BN = 256 only.
+// chain (models/line_transformer.py:157-166,176-183,245-246) is one launch instead of three.  BN = 256 only.
 constexpr int CHAIN_MAX_OPS = 4;
 struct GemmChainArgs {
   GemmImgArgs op[CHAIN_MAX_OPS];
   int n_ops, m_tiles;
 };
 
-__global__ void __launch_bounds__(320, 1) gemm_chain_kernel(const __grid_constant__ GemmChainArgs c) {
-  constexpr int BN = 256;
-  using Cfg = GemmImgCfg<BN>;
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t raw = ptx::smem_u32(smem_raw);
-  uint8_t* smem = smem_raw + ((1024u - (raw & 1023u)) & 1023u);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::OFF_BAR);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + Cfg::STAGES;
-  uint64_t* acc_full = bars + 2 * Cfg::STAGES;
-  uint64_t* acc_empty = acc_full + 2;
-  uint64_t* op_done = acc_empty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(op_done + 1);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  pdl_launch_dependents();
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < Cfg::STAGES; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      ptx::mbar_init(&acc_full[b], 1);
-      ptx::mbar_init(&acc_empty[b], 8);
-    }
-    ptx::mbar_init(op_done, 8);
-    ptx::fence_mbar_init();
-  }
-  if (warp == 1) {
-    ptx::tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
-    ptx::tmem_relinquish();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-  if (tid == 0) LTR_DBG_STAMP(110);
-
-  if (warp == 0) {
-    // ---------------------------------------------------------------- TMA producer
-    if (lane == 0) {
-      uint32_t it = 0, dep = 0;
-      for (int mt = blockIdx.x; mt < c.m_tiles; mt += gridDim.x) {
-        for (int o = 0; o < c.n_ops; ++o) {
-          const GemmImgArgs& p = c.op[o];
-          if (o > 0) {   // A of this op = output of op o-1 for this m-tile: wait until it is written and visible
-            ptx::mbar_wait(op_done, dep & 1);
-            ++dep;
-            if (dep < 8) LTR_DBG_STAMP(100 + dep);
-          }
-          const int nk = p.W.K / 64;
-          const uint8_t* whi = reinterpret_cast<const uint8_t*>(p.W.hi);
-          const uint8_t* wlo = reinterpret_cast<const uint8_t*>(p.W.lo);
-          for (int nb = 0; nb < p.n_blks; ++nb)
-            for (int kb = 0; kb < nk; ++kb, ++it) {
-              const int s = it % Cfg::STAGES;
-              const uint32_t ph = (it / Cfg::STAGES) & 1;
-              ptx::mbar_wait(&empty[s], ph ^ 1);
-              uint8_t* st = smem + s * Cfg::STAGE;
-              const size_t aoff = ((size_t)mt * p.A.kblocks + p.a_kb0 + kb) * IMG_TILE_ELEMS;
-              const size_t woff = ((size_t)kb * (p.W.N / 8) + (size_t)nb * (BN / 8)) * 1024;
-              ptx::mbar_arrive_expect_tx(&full[s], Cfg::STAGE);
-              ptx::bulk_g2s(st, p.A.hi + aoff, Cfg::A_TILE, &full[s]);
-              ptx::bulk_g2s(st + Cfg::A_TILE, p.A.lo + aoff, Cfg::A_TILE, &full[s]);
-              ptx::bulk_g2s(st + 2 * Cfg::A_TILE, whi + woff, Cfg::W_TILE, &full[s]);
-              ptx::bulk_g2s(st + 2 * Cfg::A_TILE + Cfg::W_TILE, wlo + woff, Cfg::W_TILE, &full[s]);
-            }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ---------------------------------------------------------------- MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc = ptx::make_idesc_bf16_f32(128, BN);
-      uint32_t it = 0, tl = 0;
-      for (int mt = blockIdx.x; mt < c.m_tiles; mt += gridDim.x)
-        for (int o = 0; o < c.n_ops; ++o) {
-          const int nk = c.op[o].W.K / 64, n_blks = c.op[o].n_blks;
-          for (int nb = 0; nb < n_blks; ++nb, ++tl) {
-            const uint32_t buf = tl & 1, aph = (tl >> 1) & 1;
-            ptx::mbar_wait(&acc_empty[buf], aph ^ 1);
-            ptx::tc_fence_after();
-            if (tl < 10) LTR_DBG_STAMP(40 + tl * 4);
-            const uint32_t d_tmem = tmem_base + buf * BN;
-            for (int kb = 0; kb < nk; ++kb, ++it) {
-              const int s = it % Cfg::STAGES;
-              const uint32_t ph = (it / Cfg::STAGES) & 1;
-              ptx::mbar_wait(&full[s], ph);
-              ptx::tc_fence_after();
-              if (tl < 10 && kb == 0) LTR_DBG_STAMP(41 + tl * 4);
-              const uint32_t a_hi = ptx::smem_u32(smem + s * Cfg::STAGE);
-              const uint32_t a_lo = a_hi + Cfg::A_TILE;
-              const uint32_t w_hi = a_hi + 2 * Cfg::A_TILE;
-              const uint32_t w_lo = w_hi + Cfg::W_TILE;
-#pragma unroll
-              for (int k16 = 0; k16 < 4; ++k16) {
-                const uint32_t ko = k16 * 32;
-                const uint64_t dah = ptx::make_sw128_kmajor_desc(a_hi + ko, 1024);
-                const uint64_t dal = ptx::make_sw128_kmajor_desc(a_lo + ko, 1024);
-                const uint64_t dwh = ptx::make_sw128_kmajor_desc(w_hi + ko, 1024);
-                const uint64_t dwl = ptx::make_sw128_kmajor_desc(w_lo + ko, 1024);
-                ptx::umma_bf16(d_tmem, dal, dwh, idesc, (kb | k16) != 0);
-                ptx::umma_bf16(d_tmem, dah, dwl, idesc, 1);
-                ptx::umma_bf16(d_tmem, dah, dwh, idesc, 1);
-              }
-              ptx::umma_commit(&empty[s]);
-            }
-            ptx::umma_commit(&acc_full[buf]);
-            if (tl < 10) LTR_DBG_STAMP(42 + tl * 4);
-          }
-        }
-    }
-  } else {
-    // ---------------------------------------------------------------- epilogue (8 warps)
-    const int q = warp & 3;
-    const int half = (warp - 2) >> 2;
-    float* stg = reinterpret_cast<float*>(smem + Cfg::OFF_STG + (warp - 2) * Cfg::STG_WARP);
-    uint8_t* stgb = reinterpret_cast<uint8_t*>(stg);
-    uint32_t tl = 0;
-    for (int mt = blockIdx.x; mt < c.m_tiles; mt += gridDim.x)
-      for (int o = 0; o < c.n_ops; ++o) {
-        const GemmImgArgs& p = c.op[o];
-        for (int nb = 0; nb < p.n_blks; ++nb, ++tl) {
-          const uint32_t buf = tl & 1, aph = (tl >> 1) & 1;
-          ptx::mbar_wait(&acc_full[buf], aph);
-          ptx::tc_fence_after();
-          const uint32_t tacc = tmem_base + ((uint32_t)(q * 32) << 16) + buf * BN;
-          if (tl < 10 && warp == 2 && lane == 0) LTR_DBG_STAMP(80 + tl);
-          if (p.norm != NORM_NONE)
-            epi_norm_tile(p, tacc, mt, q, half, lane, tl, stg, stgb, reinterpret_cast<float*>(smem + Cfg::OFF_XCH));
-          else
-            epi_plain_tile<BN>(p, tacc, mt, nb, q, half, lane, stg, stgb);
-          ptx::tc_fence_before();
-          __syncwarp();
-          if (tl < 10 && warp == 2 && lane == 0) LTR_DBG_STAMP(43 + tl * 4);
-          if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
-        }
-        if (o + 1 < c.n_ops) {
-          // everything this warp stored for op o (generic proxy, global) must be visible to the bulk copies
-          // (async proxy) the producer issues for op o+1: device-scope fence + proxy fence, then signal
-          __threadfence();
-          ptx::fence_proxy_async_all();
-          __syncwarp();
-          if (lane == 0) ptx::mbar_arrive(op_done);
-        }
-      }
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 1) ptx::tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
-}
-
-// ---------------------------------------------------------------- CTA-pair variant of the chained GEMM (tcgen05 cta_group::2)
-// With 128 x 256 tiles one SM has to pull 96 KB of operands (A 32 KB + W 64 KB, split-bf16) per 64-deep k-block
-// against 12 x 128 = 1536 tensor cycles: 62.5 B/cycle/SM, more than the ~43 B/cycle/SM the L2 -> SM path
-// delivers (measured: 12.7 TB/s aggregate), so the single-CTA engine tops out near 0.65 of the tensor pipe.
+// The chain runs on CTA pairs (tcgen05 cta_group::2).  With 128 x 256 tiles one SM has to pull 96 KB of operands
+// (A 32 KB + W 64 KB, split-bf16) per 64-deep k-block against 12 x 128 = 1536 tensor cycles: 62.5 B/cycle/SM, more
+// than the ~43 B/cycle/SM the L2 -> SM path delivers (measured: 12.7 TB/s aggregate), so a single-CTA engine
+// (gemm_img_kernel) tops out near 0.65 of the tensor pipe.
 // A CTA pair (cluster of 2 on one TPC) shares every W tile: each CTA loads only HALF of it (128 of the 256
 // n-rows) plus its own 128-row A tile, and one tcgen05.mma.cta_group::2 of the leader CTA multiplies
 // M = 256 (128 rows per CTA) x N = 256: 64 KB per SM per k-block = 41.7 B/cycle/SM.
@@ -1303,12 +1147,12 @@ inline int launch_gemm_img(const GemmImgArgs& a, cudaStream_t s, int bn_hint = 0
   return launch_gemm_img_bn<128>(a, s);
 }
 
-// Chain of row-local layers in one launch (see gemm_chain_kernel).  Every op: N % 256 == 0, plain A
-// (no block-diagonal slices); op i+1 must read what op i writes for the same rows only.
-// pair = true: CTA-pair engine (gemm_chain2_kernel); the images it reads (A, residual, addend) must be padded to 256 rows
-// (ltr_api.cu carve does).  O may be padded to 128 rows only (the caller's descriptor tile image): the store warp drops
-// the output of the phantom tile an odd tile count gives the last cluster.
-inline int launch_gemm_chain(const GemmImgArgs* ops, int n_ops, cudaStream_t s, bool pair = false) {
+// Chain of row-local layers in one launch of gemm_chain2_kernel (see "chained GEMMs" above).  Every op: N % 256 == 0,
+// plain A (no block-diagonal slices); op i+1 must read what op i writes for the same rows only.  The images the chain
+// reads (A, residual, addend) must be padded to 256 rows (ltr_api.cu carve does).  O may be padded to 128 rows only
+// (the caller's descriptor tile image): the store warp drops the output of the phantom tile an odd tile count gives the
+// last cluster.
+inline int launch_gemm_chain(const GemmImgArgs* ops, int n_ops, cudaStream_t s) {
   if (n_ops < 1 || n_ops > CHAIN_MAX_OPS) return set_error(-1, "gemm_chain: 1..4 ops");
   if (ops[0].M <= 0) return 0;
   GemmChainArgs c{};
@@ -1326,30 +1170,22 @@ inline int launch_gemm_chain(const GemmImgArgs* ops, int n_ops, cudaStream_t s, 
     if ((a.R && a.Rimg.hi) || (a.nadd && a.NaddImg.hi) || ((a.nadd || a.NaddImg.hi) && a.norm == NORM_NONE) ||
         (a.NaddImg.hi && (a.nadd_kb0 < 0 || a.nadd_kb0 + a.W.N / 64 > a.NaddImg.kblocks)))
       return set_error(-1, "gemm_chain: residual / addend given twice, addend without a row norm, or its k-blocks exceed the image");
-    // op i > 0 reads, k-block for k-block, what op i-1 wrote for the same rows (the kernels' dependency rule)
+    // op i > 0 reads, k-block for k-block, what op i-1 wrote for the same rows (the kernel's dependency rule)
     if (i > 0 && (a.A.hi != ops[i - 1].O.hi || a.a_kb0 != ops[i - 1].o_kb0 || a.W.K > ops[i - 1].W.N))
       return set_error(-1, "gemm_chain: op i must consume the image op i-1 writes (same k-blocks)");
     a.m_tiles = c.m_tiles;
     a.n_blks = a.W.N / 256;
     c.op[i] = a;
   }
-  if (pair) {
-    using Cfg = GemmPairCfg;
-    LTR_CUDA_TRY(ensure_dynamic_smem(gemm_chain2_kernel, Cfg::SMEM));
-    const int clusters = std::min((c.m_tiles + 1) / 2, device_sm_count() / 2);
-    LaunchScope ls(KC_LINEAR, s);
-    const bool traced = dbg_chain_sel() >= 0 && dbg_chain_cnt()++ == dbg_chain_sel();
-    static const int k_on = 1, k_off = 0;
-    if (traced) cudaMemcpyToSymbolAsync(g_dbg_on, &k_on, sizeof(int), 0, cudaMemcpyHostToDevice, s);
-    LTR_CUDA_TRY(launch_pdl(gemm_chain2_kernel, dim3(2 * clusters), dim3(Cfg::THREADS), Cfg::SMEM, s, c));   // __cluster_dims__(2,1,1)
-    if (traced) cudaMemcpyToSymbolAsync(g_dbg_on, &k_off, sizeof(int), 0, cudaMemcpyHostToDevice, s);
-    return 0;
-  }
-  using Cfg = GemmImgCfg<256>;
-  LTR_CUDA_TRY(ensure_dynamic_smem(gemm_chain_kernel, Cfg::SMEM));
-  const int grid = c.m_tiles < device_sm_count() ? c.m_tiles : device_sm_count();
+  using Cfg = GemmPairCfg;
+  LTR_CUDA_TRY(ensure_dynamic_smem(gemm_chain2_kernel, Cfg::SMEM));
+  const int clusters = std::min((c.m_tiles + 1) / 2, device_sm_count() / 2);
   LaunchScope ls(KC_LINEAR, s);
-  LTR_CUDA_TRY(launch_pdl(gemm_chain_kernel, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM, s, c));
+  const bool traced = dbg_chain_sel() >= 0 && dbg_chain_cnt()++ == dbg_chain_sel();
+  static const int k_on = 1, k_off = 0;
+  if (traced) cudaMemcpyToSymbolAsync(g_dbg_on, &k_on, sizeof(int), 0, cudaMemcpyHostToDevice, s);
+  LTR_CUDA_TRY(launch_pdl(gemm_chain2_kernel, dim3(2 * clusters), dim3(Cfg::THREADS), Cfg::SMEM, s, c));   // __cluster_dims__(2,1,1)
+  if (traced) cudaMemcpyToSymbolAsync(g_dbg_on, &k_off, sizeof(int), 0, cudaMemcpyHostToDevice, s);
   return 0;
 }
 

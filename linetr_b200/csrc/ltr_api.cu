@@ -15,7 +15,6 @@
 #include "gemm_img.cuh"
 #include "token_fused.cuh"
 #include "sig_attention_tc.cuh"
-#include "sig_attention_img.cuh"
 #include "tokenizer_kernels.cuh"
 #include "match_kernels.cuh"
 #include "match_tc.cuh"
@@ -58,10 +57,17 @@ struct Lin {
   TcWeight tw;
 };
 
-struct MlpTail {  // positional encoder: narrow head + the two wide layers (128->256 relu, 256->256)
-  SmallMlpWeights head;
-  Lin l2;           // 32 -> 64 as a tensor-core image with K zero-padded to one 64-wide k-block (token stage)
+// Positional encoders: 3 (token) or 5 (line) inputs -> 32 -> 64 -> 128 -> 256 -> 256, ReLU after all but the last
+// layer.  Each holds exactly what its kernels read.
+struct TokenPosWeights {  // token stage (token_fused_kernel)
+  const float *w1, *b1;   // 3 -> 32 in fp32
+  Lin l2;                 // 32 -> 64 with K zero-padded to one 64-wide k-block
   Lin l3, l4, l5;
+};
+
+struct LinePosWeights {   // line stage: narrow head (small_mlp_kernel), then the two wide layers
+  SmallMlpWeights head;   // 5 -> 32 -> 64 -> 128 in fp32
+  Lin l4, l5;
 };
 
 struct SigLayer {
@@ -78,7 +84,8 @@ struct LtrModel {
   float* arena = nullptr;
   uint16_t* tc_arena = nullptr;
   size_t arena_floats = 0;
-  ltr::MlpTail wpe{}, lpe{};
+  ltr::TokenPosWeights wpe{};
+  ltr::LinePosWeights lpe{};
   float *U = nullptr, *s_cls = nullptr, *cls = nullptr;
   ltr::Lin wv, wfc, w1, w2, wf;  // wv: 4 heads of [64,256]; wfc bias includes the CLS residual
   float *ln1g = nullptr, *ln1b = nullptr, *ln2g = nullptr, *ln2b = nullptr;
@@ -100,27 +107,23 @@ struct HostPack {
     for (size_t i = 0; i < v.size(); ++i) buf[off + i] = (float)v[i];
     return off;
   }
-  // wide layer [N,K]: bias + tensor-core image.  `groups` > 1 packs row groups of N/groups
-  // rows as independent matrices.
-  LinOff add_lin(const std::vector<double>& W, const std::vector<double>& b, int N, int K, int groups = 1) {
+  // wide layer [N,K]: bias + tensor-core image
+  LinOff add_lin(const std::vector<double>& W, const std::vector<double>& b, int N, int K) {
     LinOff o{add(b), 0, N, K};
     size_t off = (tc.size() + 511) / 512 * 512;  // 1024-byte alignment
     tc.resize(off + 2 * (size_t)N * K);
-    const int gn = N / groups;
-    for (int g = 0; g < groups; ++g)
-      pack_tc_weight(W.data() + (size_t)g * gn * K, gn, K, tc.data() + off + (size_t)g * gn * K,
-                     tc.data() + off + (size_t)N * K + (size_t)g * gn * K);
+    pack_tc_weight(W.data(), N, K, tc.data() + off, tc.data() + off + (size_t)N * K);
     o.tc = off;
     return o;
   }
 };
 
-static Lin bind_lin(const LinOff& o, float* fbase, uint16_t* tbase, int groups = 1) {
+static Lin bind_lin(const LinOff& o, float* fbase, uint16_t* tbase) {
   Lin l;
   l.b = fbase + o.b;
   l.tw.hi = reinterpret_cast<const __nv_bfloat16*>(tbase + o.tc);
   l.tw.lo = reinterpret_cast<const __nv_bfloat16*>(tbase + o.tc + (size_t)o.N * o.K);
-  l.tw.N = o.N / groups;
+  l.tw.N = o.N;
   l.tw.K = o.K;
   return l;
 }
@@ -160,43 +163,47 @@ static bool fold_layer(const TensorMap& tm, const std::string& conv, const std::
   return true;
 }
 
-struct MlpOffsets { size_t w[3], b[3]; LinOff l2, l3, l4, l5; };
-
-static bool pack_pos_encoder(const TensorMap& tm, const std::string& prefix, int in, HostPack& hp, MlpOffsets& off,
-                             std::string& err) {
+// The five layers of a positional encoder (models/line_transformer.py:9-20), eval-BatchNorm folded into the first four.
+static bool fold_pos_encoder(const TensorMap& tm, const std::string& prefix, int in, std::vector<double> (&W)[5],
+                             std::vector<double> (&b)[5], std::string& err) {
   const int ch[6] = {in, 32, 64, 128, 256, 256};
   for (int l = 0; l < 5; ++l) {
-    std::string conv = prefix + "." + std::to_string(3 * l);
-    std::string bn = (l < 4) ? prefix + "." + std::to_string(3 * l + 1) : std::string();
-    std::vector<double> W, b;
-    if (!fold_layer(tm, conv, bn, ch[l + 1], ch[l], W, b, err)) return false;
-    if (l < 3) {
-      off.w[l] = hp.add(W);
-      off.b[l] = hp.add(b);
-      if (l == 1) {   // 32 -> 64 also as a tensor-core image, K padded to 64
-        std::vector<double> Wp((size_t)64 * 64, 0.0);
-        for (int o = 0; o < 64; ++o)
-          for (int i = 0; i < 32; ++i) Wp[(size_t)o * 64 + i] = W[(size_t)o * 32 + i];
-        off.l2 = hp.add_lin(Wp, b, 64, 64);
-      }
-      if (l == 2) off.l3 = hp.add_lin(W, b, ch[l + 1], ch[l]);  // 64 -> 128 also as a tensor-core image
-    } else if (l == 3) {
-      off.l4 = hp.add_lin(W, b, ch[l + 1], ch[l]);
-    } else {
-      off.l5 = hp.add_lin(W, b, ch[l + 1], ch[l]);
-    }
+    const std::string conv = prefix + "." + std::to_string(3 * l);
+    const std::string bn = (l < 4) ? prefix + "." + std::to_string(3 * l + 1) : std::string();
+    if (!fold_layer(tm, conv, bn, ch[l + 1], ch[l], W[l], b[l], err)) return false;
   }
   return true;
 }
 
-static void bind_mlp(MlpTail& m, float* base, uint16_t* tbase, const MlpOffsets& o) {
-  m.head.w1 = base + o.w[0]; m.head.b1 = base + o.b[0];
-  m.head.w2 = base + o.w[1]; m.head.b2 = base + o.b[1];
-  m.head.w3 = base + o.w[2]; m.head.b3 = base + o.b[2];
-  m.l2 = bind_lin(o.l2, base, tbase);
-  m.l3 = bind_lin(o.l3, base, tbase);
-  m.l4 = bind_lin(o.l4, base, tbase);
-  m.l5 = bind_lin(o.l5, base, tbase);
+struct TokenPosOff { size_t w1, b1; LinOff l2, l3, l4, l5; };
+
+static bool pack_token_pos(const TensorMap& tm, HostPack& hp, TokenPosOff& off, std::string& err) {
+  std::vector<double> W[5], b[5];
+  if (!fold_pos_encoder(tm, "klenc.word_position_enc.encoder", 3, W, b, err)) return false;
+  off.w1 = hp.add(W[0]);
+  off.b1 = hp.add(b[0]);
+  std::vector<double> W2((size_t)64 * 64, 0.0);
+  for (int o = 0; o < 64; ++o)
+    for (int i = 0; i < 32; ++i) W2[(size_t)o * 64 + i] = W[1][(size_t)o * 32 + i];
+  off.l2 = hp.add_lin(W2, b[1], 64, 64);
+  off.l3 = hp.add_lin(W[2], b[2], 128, 64);
+  off.l4 = hp.add_lin(W[3], b[3], 256, 128);
+  off.l5 = hp.add_lin(W[4], b[4], 256, 256);
+  return true;
+}
+
+struct LinePosOff { size_t w[3], b[3]; LinOff l4, l5; };
+
+static bool pack_line_pos(const TensorMap& tm, HostPack& hp, LinePosOff& off, std::string& err) {
+  std::vector<double> W[5], b[5];
+  if (!fold_pos_encoder(tm, "klenc.line_position_enc.encoder", 5, W, b, err)) return false;
+  for (int l = 0; l < 3; ++l) {
+    off.w[l] = hp.add(W[l]);
+    off.b[l] = hp.add(b[l]);
+  }
+  off.l4 = hp.add_lin(W[3], b[3], 256, 128);
+  off.l5 = hp.add_lin(W[4], b[4], 256, 256);
+  return true;
 }
 
 static cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
@@ -212,7 +219,7 @@ struct EncodeWs {
   int64_t bytes;
 };
 
-static EncodeWs carve(const LtrModel* m, int n_lines, int T, char* base) {
+static EncodeWs carve(const LtrModel* m, int n_lines, char* base) {
   EncodeWs w{};
   int64_t off = 0;
   auto take = [&](int64_t bytes) {
@@ -229,7 +236,6 @@ static EncodeWs carve(const LtrModel* m, int n_lines, int T, char* base) {
     a.kblocks = K / 64;
     return a;
   };
-  (void)T;
   const int64_t R = n_lines;
   w.z = takei(R, 1024);
   w.ctx = takei(R, 256);
@@ -274,7 +280,7 @@ static int gemm(const Lin& L, const ActImg& A, int a_kb0, int M, int act, cudaSt
 }
 
 // Batches with at least this many 128-row tiles run the row-local GEMMs of a signature layer as ONE chained
-// launch (gemm_chain_kernel); smaller ones keep one launch per layer, which spreads the n-blocks of the few
+// launch (gemm_chain2_kernel); smaller ones keep one launch per layer, which spreads the n-blocks of the few
 // m-tiles over more SMs.  LTR_CHAIN_MIN_TILES overrides (0 = never chain).
 static int chain_min_tiles() {
   static const int v = [] {
@@ -283,37 +289,18 @@ static int chain_min_tiles() {
   }();
   return v;
 }
-// LTR_ATTN_IMG=1 runs uniform 128-line batches on the per-image pipelined attention kernel (sig_attention_img.cuh).
-// Off by default: measured 33.4 us per launch against 25.4 us for the general kernel (profiles/r2_attention_img.md).
-static bool attn_img() {
-  static const bool v = [] {
-    const char* e = std::getenv("LTR_ATTN_IMG");
-    return e ? std::atoi(e) != 0 : false;
-  }();
-  return v;
-}
-// LTR_GEMM_PAIR=0 runs the chains on the single-CTA engine instead of the CTA-pair (cta_group::2) one.
-static bool gemm_pair() {
-  static const bool v = [] {
-    const char* e = std::getenv("LTR_GEMM_PAIR");
-    return e ? std::atoi(e) != 0 : true;
-  }();
-  return v;
-}
 
-template <bool TOKEN>
 static int launch_small_mlp(const SmallMlpWeights& w, const float* in0, const float* in1, const float* in2, ActImg out,
                             int rows, float width, float height, cudaStream_t s) {
   if (rows <= 0) return 0;
-  constexpr int IN = TOKEN ? 3 : 5;
-  const int smem = (int)sizeof(SmallMlpSmem<IN>);
-  LTR_CUDA_TRY(ensure_dynamic_smem(small_mlp_kernel<TOKEN>, smem));
+  const int smem = (int)sizeof(SmallMlpSmem);
+  LTR_CUDA_TRY(ensure_dynamic_smem(small_mlp_kernel, smem));
   const int groups = cdiv(rows, SM_ROWS);
   int grid = cdiv(groups, SM_WARPS);
   if (grid > 148 * 3) grid = 148 * 3;
   const float scale = fmaxf(width, height) * 0.7f;
   LaunchScope ls(KC_SMALL_MLP, s);
-  LTR_CUDA_TRY(launch_pdl(small_mlp_kernel<TOKEN>, dim3(grid), dim3(SM_WARPS * 32), (size_t)smem, s, w, in0, in1, in2, out, rows,
+  LTR_CUDA_TRY(launch_pdl(small_mlp_kernel, dim3(grid), dim3(SM_WARPS * 32), (size_t)smem, s, w, in0, in1, in2, out, rows,
                           width / 2.f, height / 2.f, scale));
   return 0;
 }
@@ -341,7 +328,7 @@ static int encode_impl(LtrModel* m, const LtrEncodeInput& in, float* out_cf, flo
   {
     TokenFusedArgs a{};
     a.pnt = in.pnt; a.score = in.score; a.desc = in.desc;
-    a.w1 = m->wpe.head.w1; a.b1 = m->wpe.head.b1; a.b2 = m->wpe.head.b2;
+    a.w1 = m->wpe.w1; a.b1 = m->wpe.b1; a.b2 = m->wpe.l2.b;
     a.W2 = m->wpe.l2.tw; a.W3 = m->wpe.l3.tw; a.W4 = m->wpe.l4.tw; a.W5 = m->wpe.l5.tw;
     a.b3 = m->wpe.l3.b; a.b4 = m->wpe.l4.b; a.b5 = m->wpe.l5.b;
     a.U = m->U; a.s_cls = m->s_cls; a.cls = m->cls;
@@ -355,8 +342,7 @@ static int encode_impl(LtrModel* m, const LtrEncodeInput& in, float* out_cf, flo
   const bool chain = chain_min_tiles() > 0 && cdiv(R, 128) >= chain_min_tiles() && !out_cf && !m->sig.empty();
   const bool chain_line = chain && m->cfg.d_inner % 256 == 0;
   // line positional encoder first (its output is added in the w_2 epilogue)
-  LTR_TRY(launch_small_mlp<false>(m->lpe.head, in.sublines, in.resp, in.angle, w.l128, R, in.image_width,
-                                  in.image_height, s));
+  LTR_TRY(launch_small_mlp(m->lpe.head, in.sublines, in.resp, in.angle, w.l128, R, in.image_width, in.image_height, s));
   LTR_TRY(gemm(m->lpe.l4, w.l128, 0, R, ACT_RELU, s, nullptr, 0, &w.l256, 0));
   LTR_TRY(gemm(m->lpe.l5, w.l256, 0, R, ACT_NONE, s, nullptr, 0, &w.lpos, 0));
   {
@@ -371,7 +357,7 @@ static int encode_impl(LtrModel* m, const LtrEncodeInput& in, float* out_cf, flo
     w2.norm = NORM_LAYER; w2.eps = 1e-6f; w2.ng = m->ln2g; w2.nbeta = m->ln2b; w2.NaddImg = w.lpos; w2.nadd_kb0 = 0;
     if (chain_line) {   // row-local: fc -> w_1 -> w_2 -> qkv of signature layer 0 in one launch
       GemmImgArgs ops[4] = {fc, w1, w2, gemm_args(m->sig[0].qkv, w.xm, 0, R, ACT_NONE, nullptr, 0, &w.qkv, 0)};
-      LTR_TRY(launch_gemm_chain(ops, 4, s, gemm_pair()));
+      LTR_TRY(launch_gemm_chain(ops, 4, s));
     } else {
       LTR_TRY(launch_gemm_img(fc, s, 256));
       LTR_TRY(launch_gemm_img(w1, s));
@@ -391,9 +377,8 @@ static int encode_impl(LtrModel* m, const LtrEncodeInput& in, float* out_cf, flo
   for (size_t li = 0; li < m->sig.size(); ++li) {
     const SigLayer& L = m->sig[li];
     if (!chain || (li == 0 && !chain_line)) LTR_TRY(gemm(L.qkv, w.xm, 0, R, ACT_NONE, s, nullptr, 0, &w.qkv, 0));
-    // o -> xm[:, 256:]; images of exactly 128 lines are the 128-row tiles of the qkv image: per-image pipelined kernel
-    if (!cu && in.lines_per_image == 128 && attn_img()) LTR_TRY(launch_sig_attention_img(w.qkv, w.xm, 256, in.n_images, s));
-    else LTR_TRY(launch_sig_attention_tc(w.qkv, w.xm, 256, cu, in.lines_per_image, max_l, in.n_images, s));
+    // o -> xm[:, 256:]
+    LTR_TRY(launch_sig_attention_tc(w.qkv, w.xm, 256, cu, in.lines_per_image, max_l, in.n_images, s));
     // x += delta: the running descriptor lives ONLY as the split-bf16 image xm[:, :256] (hi + lo carries
     // ~2^-17 relative precision; an fp32 copy would double the store traffic of this epilogue)
     if (chain) {
@@ -402,7 +387,7 @@ static int encode_impl(LtrModel* m, const LtrEncodeInput& in, float* out_cf, flo
       GemmImgArgs ops[3] = {gemm_args(L.mlp1, w.xm, 0, R, ACT_RELU, nullptr, 0, &w.hm, 0),
                             gemm_args(L.mlp2, w.hm, 0, R, ACT_NONE, nullptr, 0, &w.xm, 0, nullptr, 0, &w.xm, 0),
                             last ? fin : gemm_args(m->sig[li + 1].qkv, w.xm, 0, R, ACT_NONE, nullptr, 0, &w.qkv, 0)};
-      LTR_TRY(launch_gemm_chain(ops, 3, s, gemm_pair()));
+      LTR_TRY(launch_gemm_chain(ops, 3, s));
     } else {
       LTR_TRY(gemm(L.mlp1, w.xm, 0, R, ACT_RELU, s, nullptr, 0, &w.hm, 0));
       LTR_TRY(gemm(L.mlp2, w.hm, 0, R, ACT_NONE, s, nullptr, 0, &w.xm, 0, nullptr, 0, &w.xm, 0));
@@ -499,10 +484,9 @@ int ltr_create(const LtrTensor* tensors, int32_t n_tensors, const LtrConfig* cfg
   std::string err;
   HostPack hp;
   const int D = 256, DI = cfg->d_inner;
-  MlpOffsets wpe_o{}, lpe_o{};
-  if (!pack_pos_encoder(tm, "klenc.word_position_enc.encoder", 3, hp, wpe_o, err) ||
-      !pack_pos_encoder(tm, "klenc.line_position_enc.encoder", 5, hp, lpe_o, err))
-    return set_error(LTR_E_INVALID, err);
+  TokenPosOff wpe_o{};
+  LinePosOff lpe_o{};
+  if (!pack_token_pos(tm, hp, wpe_o, err) || !pack_line_pos(tm, hp, lpe_o, err)) return set_error(LTR_E_INVALID, err);
 
   // ---- descriptive layer (only the last one is live) ----
   const std::string dl = "klenc.desc_layers." + std::to_string(cfg->n_desc_layers - 1);
@@ -617,8 +601,10 @@ int ltr_create(const LtrTensor* tensors, int32_t n_tensors, const LtrConfig* cfg
   }
   float* B = m->arena;
   uint16_t* TB = m->tc_arena;
-  bind_mlp(m->wpe, B, TB, wpe_o);
-  bind_mlp(m->lpe, B, TB, lpe_o);
+  m->wpe = {B + wpe_o.w1, B + wpe_o.b1, bind_lin(wpe_o.l2, B, TB), bind_lin(wpe_o.l3, B, TB), bind_lin(wpe_o.l4, B, TB),
+            bind_lin(wpe_o.l5, B, TB)};
+  m->lpe = {{B + lpe_o.w[0], B + lpe_o.b[0], B + lpe_o.w[1], B + lpe_o.b[1], B + lpe_o.w[2], B + lpe_o.b[2]},
+            bind_lin(lpe_o.l4, B, TB), bind_lin(lpe_o.l5, B, TB)};
   m->U = B + oU; m->s_cls = B + oS; m->cls = B + oC;
   m->wv = bind_lin(oWv, B, TB);
   m->wfc = bind_lin(oWfc, B, TB);
@@ -644,7 +630,7 @@ void ltr_destroy(LtrModel* m) {
 int64_t ltr_encode_workspace_bytes(const LtrModel* m, int32_t n_images, int32_t n_lines, int32_t n_tokens) {
   (void)n_images;
   if (!m || n_lines < 0 || n_tokens < 1) return set_error(LTR_E_INVALID, "ltr_encode_workspace_bytes: bad argument");
-  return carve(m, n_lines, n_tokens, nullptr).bytes + 256;
+  return carve(m, n_lines, nullptr).bytes + 256;
 }
 
 int64_t ltr_desc_tiles_bytes(int32_t n_lines) {
@@ -672,7 +658,7 @@ int ltr_encode(LtrModel* m, const LtrEncodeInput* in, const LtrEncodeOutput* out
     return set_error(LTR_E_INVALID, "ltr_encode: desc_tiles must be 16-byte aligned");
   LTR_CUDA_TRY(cudaSetDevice(m->device));
   char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<int64_t>(workspace), 256));
-  EncodeWs w = carve(m, in->n_lines, in->n_tokens, base);
+  EncodeWs w = carve(m, in->n_lines, base);
   if (!workspace || (base - (char*)workspace) + w.bytes > workspace_bytes)
     return set_error(LTR_E_WORKSPACE, "ltr_encode: workspace too small, need " + std::to_string(w.bytes + 256));
   return encode_impl(m, *in, out->desc_cf, out->desc_rows, out->desc_tiles, w, as_stream(stream));

@@ -1,13 +1,12 @@
 """The chained line-stage GEMM engine against the numpy oracle at production batch sizes.
 
 `ltr_encode` runs the row-local GEMMs of the line stage and of every signature layer as one chained launch per layer
-(gemm_chain2_kernel, CTA pairs over 256-row cluster tiles; LTR_GEMM_PAIR=0: the single-CTA gemm_chain_kernel) when the
-batch has at least `chain_min_tiles()` (96) row tiles of 128 lines and no channel-first output is asked for.  Smaller
-batches and `LineTransformer.forward` never take that path, so these tests build big batches cheaply: a few distinct
-source pairs on the host, and on the device many copies of them, each copy's lines reordered by its own seeded
-permutation.  The encoder is line-permutation-equivariant, so every row's expected descriptor is its source image's
-oracle row, and every pair's expected matches are the source pair's oracle matches, permuted.  Neighbouring tiles
-never hold the same content, so a misaddressed tile shows.
+(gemm_chain2_kernel, CTA pairs over 256-row cluster tiles) when the batch has at least `chain_min_tiles()` (96) row
+tiles of 128 lines and no channel-first output is asked for.  Smaller batches and `LineTransformer.forward` never take
+that path, so these tests build big batches cheaply: a few distinct source pairs on the host, and on the device many
+copies of them, each copy's lines reordered by its own seeded permutation.  The encoder is line-permutation-equivariant,
+so every row's expected descriptor is its source image's oracle row, and every pair's expected matches are the source
+pair's oracle matches, permuted.  Neighbouring tiles never hold the same content, so a misaddressed tile shows.
 
 Every encode is counted: the number of "linear"-class launches tells which engine ran (see LINEAR_* below).
 
@@ -413,12 +412,11 @@ def test_chained_equals_unchained():
 
 # ------------------------------------------------------------------ 7. small tile counts with the chain forced
 @pytest.mark.skipif(FORCED, reason="parent of the forced_* tests")
-@pytest.mark.parametrize("pair_engine", ["1", "0"])
-def test_small_tile_counts_on_the_chain(pair_engine):
-    """The forced_* tests in a child pytest with LTR_CHAIN_MIN_TILES=1, on the CTA-pair engine and (LTR_GEMM_PAIR=0)
-    on the single-CTA gemm_chain_kernel, which no default batch size reaches."""
+def test_small_tile_counts_on_the_chain():
+    """The forced_* tests in a child pytest with LTR_CHAIN_MIN_TILES=1: tile counts (1, 2, 3, 5, ragged, 64-line images)
+    that no default batch size runs on the chain."""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, LTR_CHAIN_MIN_TILES="1", LTR_GEMM_PAIR=pair_engine)
+    env = dict(os.environ, LTR_CHAIN_MIN_TILES="1")
     cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [
         "-m", "pytest", os.path.join("tests", "test_chain_parity.py"), "-m", "gpu", "-k", "forced",
         "-p", "no:cacheprovider", "-q"]

@@ -1,6 +1,5 @@
 """clock64 timeline of CTA 0 of the LAST chained GEMM launch of an encode (mlp1 -> mlp2 -> final_proj of
-signature layer 6; 2 + 1 + 1 tiles) - MMA issue, accumulator ready, epilogue done, op-boundary waits.
-LTR_GEMM_PAIR=0/1 selects the engine."""
+signature layer 6; 2 + 1 + 1 tiles) - MMA issue, accumulator ready, epilogue done, op-boundary waits."""
 import ctypes as C
 import os
 import sys
@@ -29,7 +28,7 @@ buf = (C.c_uint64 * 128)()
 lib.ltr_debug_trace_read(buf)
 lib.ltr_debug_trace_arm(0)
 t0 = buf[110]
-print("engine:", "pair" if os.environ.get("LTR_GEMM_PAIR", "1") != "0" else "single", f" chain launch {sel}  t0 = after pdl_wait")
+print(f"chain launch {sel}  t0 = after pdl_wait")
 names = {0: ["fc+LN (K256)", "w1 nb0 (K256)", "w1 nb1 (K256)", "w2+LN (K512)", "qkv nb0 (K256)", "qkv nb1", "qkv nb2"],
          7: ["mlp1 nb0 (K512)", "mlp1 nb1 (K512)", "mlp2 (K512)", "final (K256, norm)"]}.get(
     sel, ["mlp1 nb0 (K512)", "mlp1 nb1 (K512)", "mlp2 (K512)", "qkv nb0 (K256)", "qkv nb1 (K256)", "qkv nb2 (K256)"])
@@ -51,10 +50,3 @@ for d in (1, 2, 3):
     if buf[100 + d]:
         print(f"producer: op boundary {d} passed at +{buf[100 + d] - t0}")
 print(f"kernel end (CTA 0 thread 0) +{buf[111] - t0}")
-
-# per-image attention kernel (last layer): MMA thread issue times and the softmax warps' progress
-a0 = buf[112]
-if a0:
-    nm = ["S0 issued", "S1 issued", "PV0 issued", "S2 issued", "PV1 issued", "S3 issued", "PV2 issued", "PV3 issued",
-          "softmax0 done", "softmax1 done", "epilogue0 done", "softmax2 done", "softmax3 done", "epilogue3 done"]
-    print("sig_attention_img CTA 0 (cycles after pdl_wait):", ", ".join(f"{n} +{buf[113 + i] - a0}" for i, n in enumerate(nm)))
