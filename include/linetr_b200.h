@@ -161,10 +161,11 @@ typedef struct {
 } LtrMatchInput;
 
 /* Multi-GPU: the path's ONE collective - every rank learns the per-pair match counts of all ranks - fused
- * into the matcher's tail kernel.  The caller owns a SYMMETRIC int32 buffer (same size on every rank, peer
+ * into the matcher's last kernel.  The caller owns a SYMMETRIC int32 buffer (same size on every rank, peer
  * mapped over NVLink, e.g. torch.distributed._symmetric_memory) laid out as
  *     counts[LTR_GATHER_SLOTS][world][n_pairs]  followed by  flags[LTR_GATHER_SLOTS][world].
- * The last thread block of the tail kernel stores this rank's n_pairs counts into row `rank` of slot `slot`
+ * The thread block of the matcher's exact kernel that completes the last pair's counts (block 0 when no
+ * decision needed the exact path) stores this rank's n_pairs counts into row `rank` of slot `slot`
  * of EVERY rank's buffer - one multimem.st per element through the NVSwitch multicast address when `mc_base`
  * is given, else plain stores through the `world` peer pointers - and then publishes flags[slot][rank] =
  * epoch the same way.  No NCCL kernel, no extra launch on the producing side; ltr_gather_wait (one tiny

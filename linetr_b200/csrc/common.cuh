@@ -38,6 +38,7 @@ enum KernelClass : int {
   KC_DESC_TILES,
   KC_MATCH_TC,
   KC_MATCH_TAIL,
+  KC_MATCH_EXACT,
   KC_COUNT
 };
 const char* kernel_class_name(int kc);

@@ -35,7 +35,7 @@ int set_error(int code, const std::string& msg) {
 const char* kernel_class_name(int kc) {
   static const char* names[KC_COUNT] = {"small_mlp", "linear", "img_convert", "sig_attention", "final_norm",
                                          "dist", "segmean", "argmin", "mutual", "token_fused",
-                                         "tokenize", "desc_tiles", "match_tc", "match_tail"};
+                                         "tokenize", "desc_tiles", "match_tc", "match_tail", "match_exact"};
   return (kc >= 0 && kc < KC_COUNT) ? names[kc] : "?";
 }
 
@@ -671,7 +671,8 @@ struct MatchPlan {
   ActImg img[2];
   uint2* slot[2];
   float* sq[2];
-  int* done;
+  ExactQueue xq;
+  int xq_tiles;         // work-list capacity in tiles
   int64_t bytes;
 };
 
@@ -707,8 +708,12 @@ static MatchPlan plan_match(const LtrMatchInput& in, char* base) {
     }
     pl.slot[s] = reinterpret_cast<uint2*>(take((int64_t)std::max(pl.total[s], 1) * 8));
     pl.sq[s] = in.dist_mode == 1 ? reinterpret_cast<float*>(take((int64_t)std::max(pl.total[s], 1) * 4)) : nullptr;
+    pl.xq.res[s] = reinterpret_cast<uint2*>(take((int64_t)std::max(pl.total[s], 1) * 8));
   }
-  pl.done = reinterpret_cast<int*>(take(256));
+  // every tail block (256 lines of one pair, rows and columns) appends at most 256 / XT_ITEMS + 1 tiles
+  pl.xq_tiles = cdiv(pl.mx[0] + pl.mx[1], 256) * P * (256 / XT_ITEMS + 1);
+  pl.xq.ctr = reinterpret_cast<int*>(take((int64_t)(XQ_HDR + 2 * P) * 4));
+  pl.xq.tiles = reinterpret_cast<ExactTile*>(take((int64_t)std::max(pl.xq_tiles, 1) * sizeof(ExactTile)));
   pl.bytes = off;
   return pl;
 }
@@ -763,33 +768,50 @@ static int run_match_tc(const LtrMatchInput& in, const LtrMatchOutput& out, cons
     ma.dist = seg ? out.dist_sub : out.dist_key;
     ma.dist_stride = seg ? (long long)pl.mx[0] * pl.mx[1] : stride_key;
     ma.counts = want_nn ? out.counts : nullptr;
-    ma.done = want_nn ? pl.done : nullptr;
+    ma.xq_ctr = want_nn ? pl.xq.ctr : nullptr;
     ma.n_pairs = P;
     LTR_CUDA_TRY(ensure_dynamic_smem(match_tc_kernel, MT_SMEM));
     LaunchScope ls(KC_MATCH_TC, s);
     LTR_CUDA_TRY(launch_pdl(match_tc_kernel, dim3(pl.tmax[0] + (both ? pl.tmax[1] : 0), P), dim3(MT_THREADS), (size_t)MT_SMEM, s, ma));
   } else if (want_nn) {
     LTR_CUDA_TRY(cudaMemsetAsync(out.counts, 0, sizeof(int) * P, s));
-    LTR_CUDA_TRY(cudaMemsetAsync(pl.done, 0, sizeof(int), s));
+    LTR_CUDA_TRY(cudaMemsetAsync(pl.xq.ctr, 0, sizeof(int) * (XQ_HDR + 2 * P), s));
   }
   if (want_nn && pl.mx[0] > 0) {
-    MatchTailArgs ta{};
-    ta.d[0] = in.desc0; ta.d[1] = in.desc1; ta.layout = in.layout;
-    ta.cu[0] = in.cu0; ta.cu[1] = in.cu1; ta.n[0] = in.n0; ta.n[1] = in.n1;
-    ta.sq[0] = pl.sq[0]; ta.sq[1] = pl.sq[1]; ta.dist_mode = in.dist_mode;
-    ta.slot[0] = pl.slot[0]; ta.slot[1] = pl.slot[1];
-    ta.thr = in.nn_thresh; ta.mutual = in.mutual;
-    ta.matches0 = out.matches0; ta.scores0 = out.scores0; ta.nn1 = out.nn1; ta.counts = out.counts;
-    ta.max0 = pl.mx[0];
-    ta.done = pl.done; ta.n_pairs = P; ta.world = 1;
+    {
+      MatchTailArgs ta{};
+      ta.cu[0] = in.cu0; ta.cu[1] = in.cu1; ta.n[0] = in.n0; ta.n[1] = in.n1;
+      ta.slot[0] = pl.slot[0]; ta.slot[1] = pl.slot[1];
+      ta.thr = in.nn_thresh; ta.mutual = in.mutual;
+      ta.matches0 = out.matches0; ta.scores0 = out.scores0; ta.nn1 = out.nn1; ta.counts = out.counts;
+      ta.max0 = pl.mx[0];
+      ta.xq = pl.xq;
+      LaunchScope ls(KC_MATCH_TAIL, s);
+      LTR_CUDA_TRY(launch_pdl(match_tail_kernel, dim3(cdiv(pl.mx[0] + (in.mutual ? pl.mx[1] : 0), 256), P), dim3(256), 0, s, ta));
+    }
+    MatchExactArgs xa{};
+    xa.d[0] = in.desc0; xa.d[1] = in.desc1; xa.layout = in.layout;
+    xa.cu[0] = in.cu0; xa.cu[1] = in.cu1; xa.n[0] = in.n0; xa.n[1] = in.n1;
+    xa.sq[0] = pl.sq[0]; xa.sq[1] = pl.sq[1]; xa.dist_mode = in.dist_mode;
+    xa.slot[0] = pl.slot[0]; xa.slot[1] = pl.slot[1];
+    xa.thr = in.nn_thresh; xa.mutual = in.mutual;
+    xa.matches0 = out.matches0; xa.scores0 = out.scores0; xa.nn1 = out.nn1; xa.counts = out.counts;
+    xa.xq = pl.xq;
+    xa.n_pairs = P; xa.world = 1;
     if (out.gather && out.gather->world > 1) {
       const LtrPeerGather& g = *out.gather;
-      ta.mc_base = reinterpret_cast<int*>(g.mc_base);
-      ta.peer_bases = reinterpret_cast<int* const*>(g.peer_bases);
-      ta.rank = g.rank; ta.world = g.world; ta.gslot = g.slot; ta.epoch = g.epoch;
+      xa.mc_base = reinterpret_cast<int*>(g.mc_base);
+      xa.peer_bases = reinterpret_cast<int* const*>(g.peer_bases);
+      xa.rank = g.rank; xa.world = g.world; xa.gslot = g.slot; xa.epoch = g.epoch;
     }
-    LaunchScope ls(KC_MATCH_TAIL, s);
-    LTR_CUDA_TRY(launch_pdl(match_tail_kernel, dim3(cdiv(pl.mx[0] + (in.mutual ? pl.mx[1] : 0), 256), P), dim3(256), 0, s, ta));
+    // persistent CTAs; the work list is known on the device only, so the grid covers the GPU
+    int dev = 0, sms = 0;
+    LTR_CUDA_TRY(cudaGetDevice(&dev));
+    LTR_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    LTR_CUDA_TRY(ensure_dynamic_smem(match_exact_kernel, XK_SMEM));
+    LaunchScope ls(KC_MATCH_EXACT, s);
+    LTR_CUDA_TRY(launch_pdl(match_exact_kernel, dim3(std::max(1, std::min(XK_CTAS_PER_SM * sms, pl.xq_tiles))), dim3(XK_THREADS),
+                            (size_t)XK_SMEM, s, xa));
   }
   return 0;
 }

@@ -1,8 +1,8 @@
 // Tensor-core descriptor matcher (K3): all-pairs distance D = 2 - 2 <a_i, b_j> on tcgen05 with the
 // row-argmin fused into the epilogue, for BOTH directions (side 0 rows vs side 1 and side 1 rows vs
 // side 0 - the second one is the column argmin the mutual check needs), a tail kernel that applies
-// threshold + mutual check + per-pair counts, and an exact fp32 re-check for decisions the
-// tensor-core arithmetic cannot make safely.
+// threshold + mutual check + per-pair counts and lists the decisions the tensor-core arithmetic cannot
+// make safely, and an exact fp32 kernel that re-takes those over the whole GPU.
 //
 // Reference: get_dist_matrix (models/line_process.py:198-201: einsum('bdn,bdm->bnm'), (2 - 2 s).clip(0)),
 // nn_matcher / nn_matcher_distmat (models/nn_matcher.py:3-43: argmin axis 1, strict '<' threshold,
@@ -12,7 +12,7 @@
 // Precision contract.  The contraction is a 3-term split-bf16 product (hi*hi + lo*hi + hi*lo, fp32
 // accumulate in TMEM): ~1e-5 absolute on a distance.  Match indices must be bit-exact, so every row
 // whose best and second-best distance are closer than MATCH_EPS, or whose best distance lies within
-// MATCH_EPS of the threshold, is recomputed by the tail kernel with fp32 FMAs in ascending k order
+// MATCH_EPS of the threshold, is recomputed by match_exact_kernel with fp32 FMAs in ascending k order
 // (the arithmetic of the round-1 FFMA matcher the golden vectors were pinned with) before any decision
 // is taken.  Exact ties therefore resolve to the lowest index exactly as np.argmin does.
 //
@@ -55,13 +55,32 @@ struct MatchSide {
   uint2* slot;           // out: per line {bits(best distance), best index | ambiguous << 31}
 };
 
+// Work list of the exact re-check: an item is one line whose tensor-core argmin cannot be trusted, a tile up to
+// XT_ITEMS items of one pair and side.  match_tail_kernel appends, match_exact_kernel takes.
+constexpr int XT_ITEMS = 32;
+struct ExactTile {
+  int pair, side, n, pad;
+  int line[XT_ITEMS];    // lines inside the pair
+};
+// counters (zeroed by match_tc_kernel, or by a memset when it does not run)
+constexpr int XQ_TILES = 0;      // tiles on the list
+constexpr int XQ_HEAD = 1;       // next tile to take
+constexpr int XQ_PAIRS = 2;      // pairs with at least one tile
+constexpr int XQ_FINISHED = 3;   // pairs whose open decisions are made (multi-GPU publication)
+constexpr int XQ_HDR = 4;        // then tiles per pair [n_pairs], finished tiles per pair [n_pairs]
+struct ExactQueue {
+  int* ctr;
+  ExactTile* tiles;      // capacity: 256 / XT_ITEMS + 1 tiles per tail block
+  uint2* res[2];         // per line of each side: {bits(exact best distance), exact best index}, items only
+};
+
 struct MatchTcArgs {
   MatchSide s[2];
   int dist_mode;         // 0: 2 - 2 s (unit descriptors, nn_matcher.py:37-38)   1: |a|^2 + |b|^2 - 2 s (evaluations/matcher.py:66-70)
   float* dist;           // optional dense output of side 0 vs side 1, pair p at p * dist_stride, row-major [n0_p, n1_p]
   long long dist_stride;
-  int* counts;           // zeroed here (the tail kernel accumulates into it)
-  int* done;             // tail-kernel block counter (last-block detection), zeroed here
+  int* counts;           // zeroed here (the tail and exact kernels accumulate into it)
+  int* xq_ctr;           // exact work-list counters (XQ_HDR + 2 n_pairs), zeroed here
   int n_pairs;
 };
 
@@ -122,7 +141,12 @@ __global__ void __launch_bounds__(MT_THREADS, 1) match_tc_kernel(MatchTcArgs p) 
   side_range(SB, pair, bb, eb);
   const int na = ea - ba, nb = eb - bb;
   if (p.counts && blockIdx.x == 0 && tid == 0) p.counts[pair] = 0;
-  if (p.done && blockIdx.x == 0 && pair == 0 && tid == 0) *p.done = 0;
+  if (p.xq_ctr && blockIdx.x == 0 && tid == 0) {
+    p.xq_ctr[XQ_HDR + pair] = 0;
+    p.xq_ctr[XQ_HDR + p.n_pairs + pair] = 0;
+    if (pair == 0)
+      for (int i = 0; i < XQ_HDR; ++i) p.xq_ctr[i] = 0;
+  }
   const bool active = rb * 128 < na && nb > 0;   // uniform per CTA
   const int n_ct = active ? (nb + 127) >> 7 : 0;
 
@@ -365,22 +389,6 @@ __global__ void __launch_bounds__(256) desc_tiles_kernel(DescTilesArgs p) {
   }
 }
 
-// ---------------------------------------------------------------- tail: exact re-check, threshold, mutual, counts
-struct MatchTailArgs {
-  const float* d[2]; int layout;   // the fp32 descriptors the tiles were made from (exact re-check)
-  const int* cu[2]; int n[2];
-  const float* sq[2];              // distance mode 1
-  int dist_mode;
-  const uint2* slot[2];
-  float thr; int mutual;
-  int* matches0; float* scores0; int* nn1; int* counts;
-  int max0;                        // max lines of side 0 per pair (row part of the grid)
-  // multi-GPU publication of `counts` (LtrPeerGather): symmetric buffer = counts[SLOTS][world][n_pairs] | flags[SLOTS][world]
-  int* done;                       // block counter for last-block detection
-  int* mc_base; int* const* peer_bases;
-  int rank, world, gslot, epoch, n_pairs;
-};
-
 constexpr int GATHER_SLOTS = 8;   // = LTR_GATHER_SLOTS
 __device__ __forceinline__ void multimem_st_u32(int* mc_addr, int v) {
   asm volatile("multimem.st.relaxed.sys.global.u32 [%0], %1;" ::"l"(mc_addr), "r"(v) : "memory");
@@ -391,95 +399,33 @@ __device__ __forceinline__ int ld_acquire_sys(const int* p) {
   return v;
 }
 
-// Exact fp32 distances of line `r` of side `sa` to every line of the other side (ascending-k fmaf chain,
-// the arithmetic of the round-1 FFMA matcher), first-minimum argmin over them; whole warp.
-__device__ __forceinline__ void exact_row(const MatchTailArgs& p, int sa, int pair_b_a, int na, int r, int pair_b_b, int nb,
-                                          float* xrow, int lane, float& best, int& bidx) {
-  const int sb = sa ^ 1;
-  const float* __restrict__ A = p.d[sa];
-  const float* __restrict__ B = p.d[sb];
-  // stage the row in shared memory (per-warp 1 KB)
-  if (p.layout == 0) {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) xrow[i * 32 + lane] = A[(size_t)(pair_b_a + r) * MT_D + i * 32 + lane];
-  } else {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) xrow[i * 32 + lane] = A[(size_t)pair_b_a * MT_D + (size_t)(i * 32 + lane) * na + r];
-  }
-  __syncwarp();
-  const float sqa = p.dist_mode == 1 ? p.sq[sa][pair_b_a + r] : 0.f;
-  best = INFINITY; bidx = 0x7fffffff;
-  for (int j = lane; j < nb; j += 32) {
-    float acc = 0.f;
-    if (p.layout == 0) {
-      const float4* __restrict__ y = reinterpret_cast<const float4*>(B + (size_t)(pair_b_b + j) * MT_D);
-#pragma unroll 8
-      for (int k = 0; k < MT_D / 4; ++k) {
-        const float4 b = y[k];
-        acc = fmaf(xrow[4 * k], b.x, acc);
-        acc = fmaf(xrow[4 * k + 1], b.y, acc);
-        acc = fmaf(xrow[4 * k + 2], b.z, acc);
-        acc = fmaf(xrow[4 * k + 3], b.w, acc);
-      }
-    } else {
-      const float* __restrict__ y = B + (size_t)pair_b_b * MT_D + j;
-#pragma unroll 8
-      for (int k = 0; k < MT_D; ++k) acc = fmaf(xrow[k], y[(size_t)k * nb], acc);
-    }
-    const float v = p.dist_mode == 1 ? fmaxf((sqa + p.sq[sb][pair_b_b + j]) - 2.f * acc, 0.f) : fmaxf(2.f - 2.f * acc, 0.f);
-    if (v < best) { best = v; bidx = j; }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bidx, o);
-    if (ov < best || (ov == best && oi < bidx)) { best = ov; bidx = oi; }
-  }
-  __syncwarp();
-}
+// ---------------------------------------------------------------- tail: threshold, mutual check, counts, exact work list
+struct MatchTailArgs {
+  const int* cu[2]; int n[2];
+  const uint2* slot[2];
+  float thr; int mutual;
+  int* matches0; float* scores0; int* nn1; int* counts;
+  int max0;                        // max lines of side 0 per pair (row part of the grid)
+  ExactQueue xq;
+};
 
-// One decision (warp-cooperative; used for the lines whose slots are flagged ambiguous): side-0 line i ->
-// matches0 / scores0 (returns keep), or side-1 line j -> nn1.
-__device__ __forceinline__ bool tail_decide_row(const MatchTailArgs& p, int i, int b0, int n0, int b1, int n1, float* xrow, int lane,
-                                                bool force_exact) {
-  const uint2 s = p.slot[0][b0 + i];
-  float v = __uint_as_float(s.x);
-  int idx = (int)(s.y & 0x7fffffffu);
-  if (force_exact || (s.y >> 31) || !(fabsf(v - p.thr) >= MATCH_EPS)) exact_row(p, 0, b0, n0, i, b1, n1, xrow, lane, v, idx);
-  bool keep = v < p.thr;   // strict '<' (nn_matcher.py:18)
-  if (keep && p.mutual) {
-    const uint2 t = p.slot[1][b1 + idx];
-    int back = (int)(t.y & 0x7fffffffu);
-    if (t.y >> 31) {
-      float bv;
-      exact_row(p, 1, b1, n1, idx, b0, n0, xrow, lane, bv, back);
-    }
-    keep = back == i;
-  }
-  if (lane == 0) {
-    p.matches0[b0 + i] = keep ? idx : -1;
-    p.scores0[b0 + i] = v;
-  }
-  return keep;
-}
-
-// grid = (ceil((max0 + max1) / 256), n_pairs), 256 threads, one line per THREAD on the fast path: items below
-// max0 decide side-0 lines (matches0 / scores0 / counts), the others publish nn1 (argmin over axis 0).
-// Lines whose tensor-core result cannot be trusted (ambiguous slot, score next to the threshold, or an
-// ambiguous partner column) go to a shared work list that the block's 8 warps then process
-// cooperatively with exact fp32 arithmetic.
+// grid = (ceil((max0 + max1) / 256), n_pairs), 256 threads, one line per thread: items below max0 decide side-0
+// lines (matches0 / scores0 / counts), the others publish nn1 (argmin over axis 0).  Lines whose tensor-core
+// argmin cannot be trusted (ambiguous slot, or a side-0 score next to the threshold) are appended to the exact
+// work list in tiles of up to XT_ITEMS lines of one pair and side; match_exact_kernel takes them.  A side-0 row
+// whose only doubt is an ambiguous partner column keeps its own tensor-core result and is left undecided: it
+// needs that column's exact argmin, and the column is on the list.
 __global__ void __launch_bounds__(256) match_tail_kernel(MatchTailArgs p) {
-  __shared__ float xrows[8][MT_D];
-  __shared__ int work[256];
-  __shared__ int n_work, n_keep;
+  __shared__ int list[2][256];
+  __shared__ int n_list[2], n_keep, tile0[2];
   pdl_launch_dependents();
   pdl_wait();
-  const int pair = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int pair = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
   int b0, e0, b1, e1;
   image_range(p.cu[0], p.n[0], pair, b0, e0);
   image_range(p.cu[1], p.n[1], pair, b1, e1);
   const int n0 = e0 - b0, n1 = e1 - b1;
-  if (tid == 0) { n_work = 0; n_keep = 0; }
+  if (tid == 0) { n_list[0] = 0; n_list[1] = 0; n_keep = 0; }
   __syncthreads();
   const int w = blockIdx.x * 256 + tid;
   bool keep = false;
@@ -493,17 +439,18 @@ __global__ void __launch_bounds__(256) match_tail_kernel(MatchTailArgs p) {
         const uint2 s = p.slot[0][b0 + i];
         const float v = __uint_as_float(s.x);
         const int idx = (int)(s.y & 0x7fffffffu);
-        bool hard = (s.y >> 31) || !(fabsf(v - p.thr) >= MATCH_EPS);
-        if (!hard) {
-          keep = v < p.thr;
+        if ((s.y >> 31) || !(fabsf(v - p.thr) >= MATCH_EPS)) {
+          list[0][atomicAdd(&n_list[0], 1)] = i;
+        } else {
+          keep = v < p.thr;   // strict '<' (nn_matcher.py:18)
+          bool defer = false;
           if (keep && p.mutual) {
             const uint2 t = p.slot[1][b1 + idx];
-            if (t.y >> 31) { hard = true; keep = false; }
-            else keep = (int)(t.y & 0x7fffffffu) == i;
+            defer = (t.y >> 31) != 0;
+            keep = !defer && (int)(t.y & 0x7fffffffu) == i;
           }
+          if (!defer) { p.matches0[b0 + i] = keep ? idx : -1; p.scores0[b0 + i] = v; }
         }
-        if (hard) work[atomicAdd(&n_work, 1)] = w;
-        else { p.matches0[b0 + i] = keep ? idx : -1; p.scores0[b0 + i] = v; }
       }
     }
   } else if (p.mutual) {
@@ -512,7 +459,7 @@ __global__ void __launch_bounds__(256) match_tail_kernel(MatchTailArgs p) {
       if (n0 == 0) p.nn1[b1 + j] = -1;
       else {
         const uint2 t = p.slot[1][b1 + j];
-        if (t.y >> 31) work[atomicAdd(&n_work, 1)] = w;
+        if (t.y >> 31) list[1][atomicAdd(&n_list[1], 1)] = j;
         else p.nn1[b1 + j] = (int)(t.y & 0x7fffffffu);
       }
     }
@@ -520,47 +467,291 @@ __global__ void __launch_bounds__(256) match_tail_kernel(MatchTailArgs p) {
   const unsigned kb = __ballot_sync(0xffffffffu, keep);
   if (lane == 0 && kb) atomicAdd(&n_keep, __popc(kb));
   __syncthreads();
-  for (int e = warp; e < n_work; e += 8) {     // exact path, one work item per warp at a time
-    const int ww = work[e];
-    if (ww < p.max0) {
-      if (tail_decide_row(p, ww, b0, n0, b1, n1, xrows[warp], lane, false) && lane == 0) atomicAdd(&n_keep, 1);
-    } else {
-      const int j = ww - p.max0;
-      float bv; int back;
-      exact_row(p, 1, b1, n1, j, b0, n0, xrows[warp], lane, bv, back);
-      if (lane == 0) p.nn1[b1 + j] = back;
+  if (tid == 0) {
+    if (n_keep) atomicAdd(&p.counts[pair], n_keep);
+    const int t0 = (n_list[0] + XT_ITEMS - 1) / XT_ITEMS, t1 = (n_list[1] + XT_ITEMS - 1) / XT_ITEMS;
+    if (t0 + t1) {
+      const int first = atomicAdd(&p.xq.ctr[XQ_TILES], t0 + t1);
+      tile0[0] = first;
+      tile0[1] = first + t0;
+      if (atomicAdd(&p.xq.ctr[XQ_HDR + pair], t0 + t1) == 0) atomicAdd(&p.xq.ctr[XQ_PAIRS], 1);
     }
   }
   __syncthreads();
-  if (tid == 0 && n_keep) atomicAdd(&p.counts[pair], n_keep);
-  if (p.world > 1) {
-    // ---- fused collective: the LAST block of the grid publishes this rank's counts to every rank over NVLink ----
-    __shared__ int is_last;
-    if (tid == 0) {
-      __threadfence();
-      is_last = atomicAdd(p.done, 1) == (int)(gridDim.x * gridDim.y) - 1;
+#pragma unroll
+  for (int sd = 0; sd < 2; ++sd) {
+    const int n = n_list[sd];
+    if (tid < n) {
+      ExactTile& t = p.xq.tiles[tile0[sd] + tid / XT_ITEMS];
+      t.line[tid % XT_ITEMS] = list[sd][tid];
+      if (tid % XT_ITEMS == 0) { t.pair = pair; t.side = sd; t.n = min(XT_ITEMS, n - tid); }
     }
-    __syncthreads();
-    if (is_last) {
-      __threadfence();
-      const long long cnt_off = ((long long)p.gslot * p.world + p.rank) * p.n_pairs;
-      const long long flag_off = (long long)GATHER_SLOTS * p.world * p.n_pairs + (long long)p.gslot * p.world + p.rank;
-      for (int i = tid; i < p.n_pairs; i += 256) {
-        const int v = __ldcg(p.counts + i);
-        if (p.mc_base) multimem_st_u32(p.mc_base + cnt_off + i, v);
-        else
-          for (int r = 0; r < p.world; ++r) p.peer_bases[r][cnt_off + i] = v;
-      }
-      __threadfence_system();
-      __syncthreads();
-      if (tid == 0) {
-        if (p.mc_base) multimem_st_u32(p.mc_base + flag_off, p.epoch);
-        else
-          for (int r = 0; r < p.world; ++r) *reinterpret_cast<volatile int*>(p.peer_bases[r] + flag_off) = p.epoch;
-        __threadfence_system();
+  }
+}
+
+// ---------------------------------------------------------------- exact re-check of the work list
+struct MatchExactArgs {
+  const float* d[2]; int layout;   // the fp32 descriptors the tiles were made from
+  const int* cu[2]; int n[2];
+  const float* sq[2];              // distance mode 1
+  int dist_mode;
+  const uint2* slot[2];
+  float thr; int mutual;
+  int* matches0; float* scores0; int* nn1; int* counts;
+  ExactQueue xq;
+  // multi-GPU publication of `counts` (LtrPeerGather): symmetric buffer = counts[SLOTS][world][n_pairs] | flags[SLOTS][world]
+  int* mc_base; int* const* peer_bases;
+  int rank, world, gslot, epoch, n_pairs;
+};
+
+constexpr int XK_THREADS = 256;
+constexpr int XK_COLS = 128;          // lines of the other side per streamed chunk
+constexpr int XK_KC = 32;             // channels per streamed chunk
+constexpr int XK_AS = MT_D + 4;       // row stride (floats) of the staged items: conflict-free float4 reads
+constexpr int XK_BS = XK_KC + 4;      // row stride of the streamed chunk
+constexpr int XK_SMEM = (XT_ITEMS * XK_AS + XK_COLS * XK_BS + 4 * XT_ITEMS * 2 + 2 * XT_ITEMS) * 4;
+constexpr int XK_CTAS_PER_SM = 2;
+
+__device__ __forceinline__ void lex_min(float& v, int& i, float ov, int oi) {
+  if (ov < v || (ov == v && oi < i)) { v = ov; i = oi; }
+}
+
+// chunk (lines c0 .. c0 + 127 of the other side, channels k0 .. k0 + 31) -> 4 float4 per thread
+__device__ __forceinline__ void xk_load_chunk(const MatchExactArgs& p, const float* __restrict__ B, int bb, int nb, int c0, int k0,
+                                              float4 (&r)[4]) {
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int f = threadIdx.x + XK_THREADS * u;
+    r[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (p.layout == 0) {   // 8 lanes read one line's 128 contiguous bytes
+      const int c = f >> 3, q = f & 7;
+      if (c0 + c < nb) r[u] = __ldg(reinterpret_cast<const float4*>(B + (size_t)(bb + c0 + c) * MT_D + k0 + 4 * q));
+    } else {               // lanes read consecutive lines of one channel
+      const int c = f & (XK_COLS - 1), q = f >> 7;
+      if (c0 + c < nb) {
+        const float* y = B + (size_t)bb * MT_D + (size_t)(k0 + 4 * q) * nb + c0 + c;
+        r[u] = make_float4(__ldg(y), __ldg(y + nb), __ldg(y + 2 * (size_t)nb), __ldg(y + 3 * (size_t)nb));
       }
     }
   }
+}
+
+__device__ __forceinline__ void xk_store_chunk(const MatchExactArgs& p, float* Bs, const float4 (&r)[4]) {
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int f = threadIdx.x + XK_THREADS * u;
+    const int c = p.layout == 0 ? f >> 3 : f & (XK_COLS - 1);
+    const int q = p.layout == 0 ? f & 7 : f >> 7;
+    *reinterpret_cast<float4*>(Bs + c * XK_BS + 4 * q) = r[u];
+  }
+}
+
+// The decisions of one pair that the tail left open, once every tile of the pair is done: side-0 rows with an
+// exact argmin or an ambiguous partner column (matches0 / scores0 / counts) and ambiguous side-1 columns (nn1).
+__device__ __forceinline__ void exact_finish_pair(const MatchExactArgs& p, int pair) {
+  int b0, e0, b1, e1;
+  image_range(p.cu[0], p.n[0], pair, b0, e0);
+  image_range(p.cu[1], p.n[1], pair, b1, e1);
+  const int n0 = e0 - b0, n1 = e1 - b1;
+  int kept = 0;
+  for (int i = threadIdx.x; i < n0; i += XK_THREADS) {
+    const uint2 s = p.slot[0][b0 + i];
+    float v = __uint_as_float(s.x);
+    int idx = (int)(s.y & 0x7fffffffu);
+    const bool hard = (s.y >> 31) || !(fabsf(v - p.thr) >= MATCH_EPS);
+    if (hard) {
+      const uint2 x = __ldcg(p.xq.res[0] + b0 + i);
+      v = __uint_as_float(x.x);
+      idx = (int)x.y;
+    }
+    bool keep = v < p.thr;   // strict '<' (nn_matcher.py:18)
+    if (keep && p.mutual) {
+      const uint2 t = p.slot[1][b1 + idx];
+      if (!hard && !(t.y >> 31)) continue;   // decided by the tail
+      const int back = (t.y >> 31) ? (int)__ldcg(p.xq.res[1] + b1 + idx).y : (int)(t.y & 0x7fffffffu);
+      keep = back == i;
+    } else if (!hard) {
+      continue;
+    }
+    p.matches0[b0 + i] = keep ? idx : -1;
+    p.scores0[b0 + i] = v;
+    kept += keep;
+  }
+  if (p.mutual)
+    for (int j = threadIdx.x; j < n1; j += XK_THREADS)
+      if (p.slot[1][b1 + j].y >> 31) p.nn1[b1 + j] = (int)__ldcg(p.xq.res[1] + b1 + j).y;
+  kept = __reduce_add_sync(0xffffffffu, kept);
+  if ((threadIdx.x & 31) == 0 && kept) atomicAdd(&p.counts[pair], kept);
+}
+
+// The rank's counts to every rank over NVLink (whole block).
+__device__ __forceinline__ void publish_counts(const MatchExactArgs& p) {
+  __threadfence();
+  const long long cnt_off = ((long long)p.gslot * p.world + p.rank) * p.n_pairs;
+  const long long flag_off = (long long)GATHER_SLOTS * p.world * p.n_pairs + (long long)p.gslot * p.world + p.rank;
+  for (int i = threadIdx.x; i < p.n_pairs; i += XK_THREADS) {
+    const int v = __ldcg(p.counts + i);
+    if (p.mc_base) multimem_st_u32(p.mc_base + cnt_off + i, v);
+    else
+      for (int r = 0; r < p.world; ++r) p.peer_bases[r][cnt_off + i] = v;
+  }
+  __threadfence_system();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (p.mc_base) multimem_st_u32(p.mc_base + flag_off, p.epoch);
+    else
+      for (int r = 0; r < p.world; ++r) *reinterpret_cast<volatile int*>(p.peer_bases[r] + flag_off) = p.epoch;
+    __threadfence_system();
+  }
+}
+
+// Persistent CTAs take tiles of the work list from an atomic queue.  A tile's items (up to 32 lines of side A)
+// stay in shared memory; the other side's descriptors stream through shared memory in chunks of 128 lines x
+// 32 channels.  Each thread owns 4 items x 4 lines of a chunk, every distance the ascending-k fmaf chain from 0
+// (the arithmetic of the round-1 FFMA matcher), so distances, minima and first-minimum indices are bit-identical
+// to a sequential fp32 evaluation.  The CTA that finishes a pair's last tile makes that pair's open decisions;
+// with several GPUs, the CTA that finishes the last such pair (or CTA 0 if the list is empty) publishes the counts.
+__global__ void __launch_bounds__(XK_THREADS, XK_CTAS_PER_SM) match_exact_kernel(MatchExactArgs p) {
+  extern __shared__ __align__(16) float xk_smem[];
+  float* As = xk_smem;                              // [XT_ITEMS][XK_AS]
+  float* Bs = As + XT_ITEMS * XK_AS;                // [XK_COLS][XK_BS]
+  float* red_v = Bs + XK_COLS * XK_BS;              // [4][XT_ITEMS] per column-group quarter
+  int* red_i = reinterpret_cast<int*>(red_v + 4 * XT_ITEMS);
+  float* s_sq = reinterpret_cast<float*>(red_i + 4 * XT_ITEMS);
+  int* s_line = reinterpret_cast<int*>(s_sq + XT_ITEMS);
+  __shared__ int s_tile, s_last, s_pub;
+  pdl_launch_dependents();
+  pdl_wait();
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int n_tiles = p.xq.ctr[XQ_TILES];
+  const int li = (lane >> 3) + 16 * (warp & 1);     // items li + 4 e, e = 0..3
+  const int cq = warp >> 1;
+  const int cg = cq * 8 + (lane & 7);               // lines c0 + cg + 32 e of each chunk
+  for (;;) {
+    if (tid == 0) s_tile = atomicAdd(&p.xq.ctr[XQ_HEAD], 1);
+    __syncthreads();
+    const int t = s_tile;
+    if (t >= n_tiles) break;
+    const ExactTile& T = p.xq.tiles[t];
+    const int pair = T.pair, sa = T.side, sb = sa ^ 1, n = T.n;
+    int ba, ea, bb, eb;
+    image_range(p.cu[sa], p.n[sa], pair, ba, ea);
+    image_range(p.cu[sb], p.n[sb], pair, bb, eb);
+    const int na = ea - ba, nb = eb - bb;
+    const float* __restrict__ A = p.d[sa];
+    const float* __restrict__ B = p.d[sb];
+    if (tid < XT_ITEMS) {
+      const int r = tid < n ? T.line[tid] : 0;
+      s_line[tid] = r;
+      s_sq[tid] = (p.dist_mode == 1 && tid < n) ? p.sq[sa][ba + r] : 0.f;
+    }
+    __syncthreads();
+    // stage the items (rows past n are zero)
+    if (p.layout == 0) {
+      for (int f = tid; f < XT_ITEMS * MT_D / 4; f += XK_THREADS) {
+        const int it = f >> 6, q = f & 63;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (it < n) v = __ldg(reinterpret_cast<const float4*>(A + (size_t)(ba + s_line[it]) * MT_D) + q);
+        *reinterpret_cast<float4*>(As + it * XK_AS + 4 * q) = v;
+      }
+    } else {
+      for (int f = tid; f < XT_ITEMS * MT_D; f += XK_THREADS) {
+        const int it = f >> 8, k = f & (MT_D - 1);
+        As[it * XK_AS + k] = it < n ? __ldg(A + (size_t)ba * MT_D + (size_t)k * na + s_line[it]) : 0.f;
+      }
+    }
+    float best[4], sqa[4];
+    int bidx[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) { best[e] = INFINITY; bidx[e] = 0x7fffffff; }
+    const bool live = 16 * (warp & 1) < n;          // warp-uniform: this warp's items exist
+    float4 pre[4];
+    xk_load_chunk(p, B, bb, nb, 0, 0, pre);
+    for (int c0 = 0; c0 < nb; c0 += XK_COLS) {
+      float acc[4][4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+#pragma unroll 1
+      for (int k0 = 0; k0 < MT_D; k0 += XK_KC) {
+        __syncthreads();                              // the previous chunk is consumed
+        xk_store_chunk(p, Bs, pre);
+        __syncthreads();
+        const int nk = k0 + XK_KC == MT_D ? 0 : k0 + XK_KC, nc = nk ? c0 : c0 + XK_COLS;
+        if (nc < nb) xk_load_chunk(p, B, bb, nb, nc, nk, pre);
+        if (live) {
+#pragma unroll
+          for (int kq = 0; kq < XK_KC / 4; ++kq) {
+            float4 a[4], b[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) a[e] = *reinterpret_cast<const float4*>(As + (li + 4 * e) * XK_AS + k0 + 4 * kq);
+#pragma unroll
+            for (int e = 0; e < 4; ++e) b[e] = *reinterpret_cast<const float4*>(Bs + (cg + 32 * e) * XK_BS + 4 * kq);
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+              for (int j = 0; j < 4; ++j) {
+                float c = acc[i][j];
+                c = fmaf(a[i].x, b[j].x, c);
+                c = fmaf(a[i].y, b[j].y, c);
+                c = fmaf(a[i].z, b[j].z, c);
+                c = fmaf(a[i].w, b[j].w, c);
+                acc[i][j] = c;
+              }
+          }
+        }
+      }
+      if (p.dist_mode == 1) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) sqa[i] = s_sq[li + 4 * i];
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {                  // ascending lines: strict '<' keeps the first minimum
+        const int c = c0 + cg + 32 * j;
+        if (c < nb) {
+          const float sqb = p.dist_mode == 1 ? p.sq[sb][bb + c] : 0.f;
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            const float v = p.dist_mode == 1 ? fmaxf((sqa[i] + sqb) - 2.f * acc[i][j], 0.f) : fmaxf(2.f - 2.f * acc[i][j], 0.f);
+            if (v < best[i]) { best[i] = v; bidx[i] = c; }
+          }
+        }
+      }
+    }
+    // first minimum over the 32 column groups: 8 lanes of a warp, then the 4 warp pairs
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+#pragma unroll
+      for (int o = 1; o < 8; o <<= 1)
+        lex_min(best[i], bidx[i], __shfl_xor_sync(0xffffffffu, best[i], o), __shfl_xor_sync(0xffffffffu, bidx[i], o));
+      if ((lane & 7) == 0) { red_v[cq * XT_ITEMS + li + 4 * i] = best[i]; red_i[cq * XT_ITEMS + li + 4 * i] = bidx[i]; }
+    }
+    __syncthreads();
+    if (tid < n) {
+      float v = red_v[tid];
+      int ix = red_i[tid];
+#pragma unroll
+      for (int g = 1; g < 4; ++g) lex_min(v, ix, red_v[g * XT_ITEMS + tid], red_i[g * XT_ITEMS + tid]);
+      p.xq.res[sa][ba + s_line[tid]] = make_uint2(__float_as_uint(v), (uint32_t)ix);
+    }
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) s_last = atomicAdd(&p.xq.ctr[XQ_HDR + p.n_pairs + pair], 1) == p.xq.ctr[XQ_HDR + pair] - 1;
+    __syncthreads();
+    if (s_last) {
+      __threadfence();
+      exact_finish_pair(p, pair);
+      if (p.world > 1) {
+        __threadfence();
+        __syncthreads();
+        if (tid == 0) s_pub = atomicAdd(&p.xq.ctr[XQ_FINISHED], 1) == p.xq.ctr[XQ_PAIRS] - 1;
+        __syncthreads();
+        if (s_pub) publish_counts(p);
+      }
+    }
+  }
+  if (p.world > 1 && n_tiles == 0 && blockIdx.x == 0) publish_counts(p);
 }
 
 // one block: wait until every rank's flag of the slot reached `epoch`, then copy the gathered counts out

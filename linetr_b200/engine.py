@@ -366,12 +366,12 @@ def gather_counts(local_counts: torch.Tensor, n_total: int, group=None, async_op
 
 class PeerCounts:
     """The path's one collective without a collective kernel: a symmetric int32 buffer (peer-mapped over
-    NVLink with torch.distributed._symmetric_memory) into which the matcher's tail kernel of every rank
+    NVLink with torch.distributed._symmetric_memory) into which the matcher's last kernel of every rank
     stores its per-pair match counts for ALL ranks - `multimem.st` through the NVSwitch multicast address
     when the allocation supports it, plain peer stores otherwise (include/linetr_b200.h: LtrPeerGather).
 
         pc = PeerCounts(n_pairs_per_rank)                            # collective: allocation + rendezvous
-        res = eng.match_packed(batch, P, 0.8, gather=pc.publish())   # counts published by the tail kernel
+        res = eng.match_packed(batch, P, 0.8, gather=pc.publish())   # counts published by the matcher
         ...                                                          # (at most GATHER_SLOTS - 2 publishes in flight)
         all_counts = pc.collect()                                    # [world * n_pairs] of the OLDEST uncollected publish
     """

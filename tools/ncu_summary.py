@@ -12,7 +12,7 @@ import subprocess
 import sys
 
 CLASS_OF = [("gemm_img", "linear"), ("gemm_chain", "linear"), ("token_fused", "token_fused"), ("sig_attention", "sig_attention"),
-            ("match_tc", "match_tc"), ("match_tail", "match_tail"), ("desc_tiles", "desc_tiles")]
+            ("match_tc", "match_tc"), ("match_tail", "match_tail"), ("match_exact", "match_exact"), ("desc_tiles", "desc_tiles")]
 
 WANT = {
     "gpu__time_duration.sum": "duration_us",

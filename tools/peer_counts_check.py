@@ -1,4 +1,4 @@
-"""Run under torchrun with >= 2 ranks (one GPU each): the fused count gather of the matcher's tail kernel
+"""Run under torchrun with >= 2 ranks (one GPU each): the fused count gather of the matcher's last kernel
 (PeerCounts: multimem.st through the NVSwitch multicast address, or peer stores) against ncclAllGather."""
 import os
 import sys
